@@ -1,4 +1,5 @@
-"""Shared test helpers: synthetic base_data directory, model construction, comparisons."""
+"""Shared test helpers: synthetic base_data directory, model construction, golden files, comparisons."""
+import ast
 import contextlib
 import os
 import tempfile
@@ -7,6 +8,8 @@ import numpy as np
 import torch
 
 from oracle import synth, torch_ref
+
+FORWARD_OUTPUTS = ("theta", "verts", "kp_2d", "kp_3d", "rotmat")
 
 
 @contextlib.contextmanager
@@ -32,6 +35,23 @@ def oracle_forward(seed, sd, x, n_layers, hidden, is_train=False, use_h36m=False
     m = torch_ref.SmplModel.synthetic(seed)
     return torch_ref.tepose_forward(sd, m, torch.as_tensor(x), n_layers, hidden, is_train=is_train,
                                     J_regressor=m.J_regressor_h36m if use_h36m else None), m
+
+
+def load_forward_golden(path):
+    """(cfg, outputs, cut) of a forward golden file (oracle/make_golden.py:save_forward).  Files of large batches keep a seeded
+    sample of each mesh (verts_idx[r]: the vertex indices kept for output row r); cut(out) reduces a forward's outputs, torch
+    tensors on any device, to what the file holds."""
+    z = np.load(path)
+    cfg = ast.literal_eval(str(z["cfg"]))
+    gold = {k: z[k] for k in FORWARD_OUTPUTS}
+    idx = torch.from_numpy(z["verts_idx"].astype(np.int64)) if "verts_idx" in z.files else None
+
+    def cut(out):
+        if idx is None:
+            return out
+        v = out["verts"]
+        return dict(out, verts=torch.gather(v, 1, idx.to(v.device)[..., None].expand(-1, -1, v.shape[-1])))
+    return cfg, gold, cut
 
 
 def aa_to_R(aa):

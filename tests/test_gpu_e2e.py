@@ -1,14 +1,12 @@
 """GPU end-to-end parity: tepose_b200.TePose (CUDA kernels through the C ABI) against the
 golden vectors produced by the unmodified reference and against the CPU oracle."""
-import ast
 import os
 
-import numpy as np
 import pytest
 import torch
 
 from oracle import synth, torch_ref
-from tests.helpers import build_product_model, compare_outputs, oracle_forward
+from tests.helpers import build_product_model, compare_outputs, load_forward_golden, oracle_forward
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
@@ -18,13 +16,11 @@ DEV = "cuda:0"
 @pytest.mark.parametrize("fname", sorted(f for f in os.listdir(GOLD) if f.startswith("fwd_")))
 @pytest.mark.parametrize("precision", ["fp32", "bf16", "fp32_tc"])
 def test_forward_against_reference_golden(fname, precision):
-    z = np.load(os.path.join(GOLD, fname))
-    cfg = ast.literal_eval(str(z["cfg"]))
+    cfg, gold, cut = load_forward_golden(os.path.join(GOLD, fname))
     model, sd = build_product_model(cfg["seed"], cfg["seqlen"], cfg["n_layers"], cfg["hidden"], precision, DEV)
     x = torch.from_numpy(synth.make_input(cfg["seed"], cfg["batch"], cfg["seqlen"])).to(DEV)
     Jr = torch_ref.SmplModel.synthetic(cfg["seed"]).J_regressor_h36m.to(DEV) if cfg.get("use_h36m") else None
-    out = model(x, is_train=cfg.get("is_train", False), J_regressor=Jr)[-1]
-    gold = {k: z[k] for k in ("theta", "verts", "kp_2d", "kp_3d", "rotmat")}
+    out = cut(model(x, is_train=cfg.get("is_train", False), J_regressor=Jr)[-1])
     if precision in ("fp32", "fp32_tc"):   # north_star: <= 1e-4 m on verts / joints in fp32 (fp32_tc: K1 / K2 as 3-term bf16 splits on tensor cores)
         errs = compare_outputs(out, gold, label=fname)
     else:                     # north_star: <= 1 mm in bf16
@@ -160,14 +156,12 @@ def test_errors_are_loud():
 @pytest.mark.parametrize("precision", ["fp32", "bf16"])
 def test_folded_forward_against_reference_golden(fname, precision):
     """fold_linear=True: heads + IEF as one pre-composed affine map (TePose.folded) -- same tolerances."""
-    z = np.load(os.path.join(GOLD, fname))
-    cfg = ast.literal_eval(str(z["cfg"]))
+    cfg, gold, cut = load_forward_golden(os.path.join(GOLD, fname))
     model, sd = build_product_model(cfg["seed"], cfg["seqlen"], cfg["n_layers"], cfg["hidden"], precision, DEV)
     model.fold_linear = True
     x = torch.from_numpy(synth.make_input(cfg["seed"], cfg["batch"], cfg["seqlen"])).to(DEV)
     Jr = torch_ref.SmplModel.synthetic(cfg["seed"]).J_regressor_h36m.to(DEV) if cfg.get("use_h36m") else None
-    out = model(x, J_regressor=Jr)[-1]
-    gold = {k: z[k] for k in ("theta", "verts", "kp_2d", "kp_3d", "rotmat")}
+    out = cut(model(x, J_regressor=Jr)[-1])
     tol = {} if precision == "fp32" else dict(vert_tol=1e-3, rot_tol=2e-3, kp2d_tol=5e-2)
     print(fname, precision, compare_outputs(out, gold, label=fname, **tol))
 

@@ -1,7 +1,6 @@
 """CPU tests of the Python host layer (packing, segment tables, job time-indexing, joint
 composition, state_dict compatibility) with the native calls emulated on CPU
 (tests/fake_native.py).  The CUDA kernels themselves are tested in the -m gpu files."""
-import ast
 import os
 
 import numpy as np
@@ -10,7 +9,7 @@ import torch
 
 from oracle import synth, torch_ref
 from tests import fake_native
-from tests.helpers import base_data_cwd, build_product_model, compare_outputs, oracle_forward
+from tests.helpers import base_data_cwd, build_product_model, compare_outputs, load_forward_golden, oracle_forward
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 CASES = [
@@ -68,15 +67,14 @@ def test_state_dict_keys_match_reference_layout():
 
 @pytest.mark.parametrize("fname", sorted(f for f in os.listdir(GOLD) if f.startswith("fwd_")))
 def test_host_layer_against_reference_golden(fname):
-    z = np.load(os.path.join(GOLD, fname))
-    cfg = ast.literal_eval(str(z["cfg"]))
+    cfg, gold, cut = load_forward_golden(os.path.join(GOLD, fname))
     model, sd = build_product_model(cfg["seed"], cfg["seqlen"], cfg["n_layers"], cfg["hidden"])
     x = synth.make_input(cfg["seed"], cfg["batch"], cfg["seqlen"])
     m = torch_ref.SmplModel.synthetic(cfg["seed"])
     with fake_native.install():
         out = model(torch.from_numpy(x), is_train=cfg.get("is_train", False),
                     J_regressor=m.J_regressor_h36m if cfg.get("use_h36m") else None)[-1]
-    compare_outputs(out, {k: z[k] for k in ("theta", "verts", "kp_2d", "kp_3d", "rotmat")}, label=fname)
+    compare_outputs(cut(out), gold, label=fname)
 
 
 def test_smpl_module_api():

@@ -1,7 +1,6 @@
 """CPU tests: the oracle against (i) golden vectors produced by the unmodified
 reference modules (oracle/make_golden.py), (ii) the independent float64 restatement,
 (iii) invariants of the un-pinned smplx boundary (SURVEY.md H9)."""
-import ast
 import os
 
 import numpy as np
@@ -9,26 +8,21 @@ import pytest
 import torch
 
 from oracle import np64, synth, torch_ref
+from tests.helpers import load_forward_golden
 
 GOLD = os.path.join(os.path.dirname(__file__), "golden")
 FWD = sorted(f for f in os.listdir(GOLD) if f.startswith("fwd_"))
 
 
-def load_case(fname):
-    z = np.load(os.path.join(GOLD, fname))
-    cfg = ast.literal_eval(str(z["cfg"]))
-    return cfg, {k: z[k] for k in ("theta", "verts", "kp_2d", "kp_3d", "rotmat")}
-
-
 @pytest.mark.parametrize("fname", FWD)
 def test_oracle_matches_reference_golden(fname):
-    cfg, gold = load_case(fname)
+    cfg, gold, cut = load_forward_golden(os.path.join(GOLD, fname))
     sd = synth.make_state_dict(cfg["seed"], cfg["n_layers"], cfg["hidden"])
     m = torch_ref.SmplModel.synthetic(cfg["seed"])
     x = torch.from_numpy(synth.make_input(cfg["seed"], cfg["batch"], cfg["seqlen"]))
-    out = torch_ref.tepose_forward(sd, m, x, cfg["n_layers"], cfg["hidden"],
-                                   is_train=cfg.get("is_train", False),
-                                   J_regressor=m.J_regressor_h36m if cfg.get("use_h36m") else None)
+    out = cut(torch_ref.tepose_forward(sd, m, x, cfg["n_layers"], cfg["hidden"],
+                                       is_train=cfg.get("is_train", False),
+                                       J_regressor=m.J_regressor_h36m if cfg.get("use_h36m") else None))
     for k, g in gold.items():
         assert out[k].shape == g.shape
         # same torch ops on the same machine class: tight, but not bitwise across CPUs
