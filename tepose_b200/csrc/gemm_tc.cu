@@ -495,6 +495,7 @@ extern "C" int tp_gemm_bf16_tc(const void* A, int a_rows, const void* W, int w_r
     TP_CHECK_ARG(sg.out && sg.m_rows > 0 && sg.n_cols > 0, "tp_gemm_bf16_tc: segment %d is empty / has no output", i);
     TP_CHECK_ARG(sg.m_start >= 0 && sg.m_start + sg.m_rows <= a_rows, "tp_gemm_bf16_tc: segment %d rows out of range", i);
     TP_CHECK_ARG(sg.n_start >= 0 && sg.n_start + sg.n_cols <= w_rows, "tp_gemm_bf16_tc: segment %d cols out of range", i);
+    TP_CHECK_ARG(sg.n_cols % 16 == 0, "tp_gemm_bf16_tc: segment %d: n_cols=%d must be a multiple of 16", i, sg.n_cols);
     TP_CHECK_ARG(!(sg.flags & TP_GEMM_OUT_BF16) || (sg.ldc % 8 == 0 && aligned16(sg.out)), "tp_gemm_bf16_tc: segment %d: bf16 output needs ldc %% 8 == 0 and 16-byte alignment", i);
     TP_CHECK_ARG(!sg.residual || (sg.ldr % 8 == 0 && aligned16(sg.residual)), "tp_gemm_bf16_tc: segment %d: residual needs ldr %% 8 == 0 and 16-byte alignment", i);
     p.seg[i] = sg;
