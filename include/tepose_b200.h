@@ -189,6 +189,26 @@ TP_API int tp_maxpool3x3s2_nhwc_bf16(const void* in, void* out, int N, int H, in
 /* mean over the HW positions of [N, HW, C] bf16 -> [N, C] fp32 (nn.AvgPool2d(7) on the 7x7 map + view, spin.py:75,139-140) */
 TP_API int tp_avgpool_nhwc_bf16(const void* in, float* out, int N, int HW, int C, void* stream);
 
+/* ------------------------------------------------------------------ demo front end: person crops on the device
+ * One row of the crop table: the box of a tracked person (lib/data_utils/_img_utils.py: get_single_image_crop_demo, bbox =
+ * centre x, centre y, width, height in pixels) in frame `frame`, enlarged by `scale` (the demo passes 1.2).  24 bytes. */
+typedef struct tp_crop {
+  int32_t frame;
+  float cx, cy, w, h;
+  float scale;
+} tp_crop;
+/* frames uint8 [F,H,W,3] RGB -> out [N,224,224,4] bf16 NHWC, channel 3 zero (the layout tp_im2col_nhwc_bf16 takes for the HMR
+ * stem).  Crop n is generate_patch_image_cv(frames[crops[n].frame], cx, cy, w, h, 224, 224, do_flip=False, scale, rot=0)
+ * (gen_trans_from_patch_cv -> cv2.getAffineTransform -> cv2.warpAffine INTER_LINEAR / BORDER_CONSTANT 0, all with cv2's
+ * double and fixed-point rounding) followed by ToTensor + Normalize(ImageNet mean / std) in fp32 and one round to bf16:
+ * bit-identical to that host pipeline (oracle/crop_ref.py).  `crops` is a DEVICE table (N <= 65535) read when the kernel
+ * runs, so a captured graph follows boxes rewritten between replays.  Outside graph capture the call reads the frame indices
+ * back (one stream synchronisation) and rejects an index outside [0, F); a captured launch that meets one writes zeros for
+ * that crop and reads no frame.  Source positions must stay within 2^20 pixels of the origin (cv2's positions are int32 in
+ * 1/1024 pixel).  crops 4-byte, out 16-byte aligned. */
+TP_API int tp_crop_normalize_bf16(const void* frames, int F, int H, int W, const tp_crop* crops, int N, void* out,
+                                  void* stream);
+
 /* ------------------------------------------------------------------ GRU recurrence (K2)
  * One direction of one torch.nn.GRU layer (lib/models/tepose.py:53-64,73,76) given the
  * input projections gi = x.W_ih^T + b_ih.  Step s (0-based) reads gi row block

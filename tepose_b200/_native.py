@@ -37,6 +37,7 @@ EXPORTS = [
     "tp_rot6d_backward", "tp_rotmat_to_angle_axis_backward", "tp_smpl_backward_workspace_bytes", "tp_smpl_backward",
     "tp_tepose_loss_workspace_bytes", "tp_tepose_loss",
     "tp_nchw_to_nhwc_bf16", "tp_im2col_nhwc_bf16", "tp_maxpool3x3s2_nhwc_bf16", "tp_avgpool_nhwc_bf16",
+    "tp_crop_normalize_bf16",
 ]
 
 vp, i32, i64, f32, sz = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
@@ -45,6 +46,10 @@ vp, i32, i64, f32, sz = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
 class GemmSeg(C.Structure):
     _fields_ = [("m_start", i32), ("m_rows", i32), ("n_start", i32), ("n_cols", i32),
                 ("out", vp), ("ldc", i64), ("bias", vp), ("flags", i32), ("ldr", i32), ("residual", vp)]
+
+
+class Crop(C.Structure):
+    _fields_ = [("frame", i32), ("cx", f32), ("cy", f32), ("w", f32), ("h", f32), ("scale", f32)]
 
 
 class GruJob(C.Structure):
@@ -78,6 +83,7 @@ _SIGNATURES = {
     "tp_im2col_nhwc_bf16": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
     "tp_maxpool3x3s2_nhwc_bf16": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
     "tp_avgpool_nhwc_bf16": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, vp]),
+    "tp_crop_normalize_bf16": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, vp, C.c_int, vp, vp]),
     "tp_device_info": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(sz)]),
     "tp_rot6d_to_rotmat": (C.c_int, [vp, vp, i64, vp]),
     "tp_rotmat_to_angle_axis": (C.c_int, [vp, vp, i64, vp]),

@@ -40,6 +40,25 @@ class Bottleneck(nn.Module):
         raise RuntimeError("tepose_b200.hmr.Bottleneck is a parameter container; call HMR.feature_extractor / HMR.forward")
 
 
+CROP = 224                     # the demo's crop_size (get_single_image_crop_demo), HMR's input size
+CROP_FIELDS = 6                # crop-table row: frame, cx, cy, w, h, scale (tp_crop, include/tepose_b200.h)
+
+
+def make_crop_table(crops, device):
+    """[N,6] rows (frame, cx, cy, w, h, scale) -> the table tp_crop_normalize_bf16 reads, on `device`: [N,6] int32 storage, the
+    frame index as int32 and the other five fields as float32 bit patterns (the 24-byte tp_crop of include/tepose_b200.h)."""
+    t = torch.as_tensor(crops, dtype=torch.float64)
+    if t.dim() != 2 or t.shape[1] != CROP_FIELDS or t.shape[0] < 1:
+        raise ValueError(f"crops must be [N,{CROP_FIELDS}] rows (frame, cx, cy, w, h, scale), got {tuple(t.shape)}")
+    frame = t[:, 0]
+    if not t.is_cuda and not torch.equal(frame, frame.round()):          # (a check of device rows would synchronise)
+        raise ValueError("crop frame indices must be integers")
+    table = torch.empty(t.shape[0], CROP_FIELDS, dtype=torch.int32, device=t.device)
+    table[:, 0] = frame.to(torch.int32)
+    table[:, 1:] = t[:, 1:].to(torch.float32).view(torch.int32)
+    return table.to(device)
+
+
 def _fold(conv: nn.Conv2d, bn: nn.BatchNorm2d, cin_pad=None):
     """conv (no bias) followed by eval-mode BatchNorm -> ([Cout, KP] bf16 weight matrix in (ky, kx, c) column order, fp32 bias)."""
     w = conv.weight.detach().double()                     # [Cout, Cin, kh, kw]
@@ -141,18 +160,30 @@ class HMR(Regressor):
         if self.training:
             raise NotImplementedError("tepose_b200.HMR implements the eval-mode feature extractor (BatchNorm folded); call .eval()")
         nv.require_cuda(x, "x")
-        pk = self.conv_packed()
-        L = nv.lib()
-        dev = x.device
         x = x.detach().contiguous().float()
         N, C, H, W = x.shape
         if C != 3:
             raise ValueError(f"HMR.feature_extractor expects [N,3,H,W] input, got {tuple(x.shape)}")
+        x4 = torch.empty(N, H, W, 4, device=x.device, dtype=torch.bfloat16)
+        nv.check(nv.lib().tp_nchw_to_nhwc_bf16(nv.ptr(x), nv.ptr(x4), N, 3, H, W, 4, nv.stream()), "tp_nchw_to_nhwc_bf16")
+        return self.features_nhwc4(x4)
+
+    @nv.device_guard
+    def features_nhwc4(self, x4):
+        """x4 [N,H,W,4] bf16 NHWC, channel 3 zero (RGB normalised as feature_extractor's input) -> [N,2048] fp32: everything of
+        feature_extractor from the stem's im2col to the average pool."""
+        if self.training:
+            raise NotImplementedError("tepose_b200.HMR implements the eval-mode feature extractor (BatchNorm folded); call .eval()")
+        nv.require_cuda(x4, "x4")
+        if x4.dim() != 4 or x4.shape[3] != 4 or x4.dtype != torch.bfloat16:
+            raise ValueError(f"HMR.features_nhwc4 expects [N,H,W,4] bf16 input, got {tuple(x4.shape)} {x4.dtype}")
+        pk = self.conv_packed()
+        L = nv.lib()
+        dev = x4.device
+        N, H, W, _ = x4.shape
         bf = lambda *s: torch.empty(*s, device=dev, dtype=torch.bfloat16)
         st = nv.stream()
         # stem: 7x7 stride-2 conv (+BN+ReLU) as im2col over RGB0 pixels, then 3x3 stride-2 max pool
-        x4 = bf(N, H, W, 4)
-        nv.check(L.tp_nchw_to_nhwc_bf16(nv.ptr(x), nv.ptr(x4), N, 3, H, W, 4, st), "tp_nchw_to_nhwc_bf16")
         Ho, Wo = (H + 6 - 7) // 2 + 1, (W + 6 - 7) // 2 + 1
         kp = pk["stem"][0].shape[1]
         cols = bf(N * Ho * Wo, kp)
@@ -197,6 +228,24 @@ class HMR(Regressor):
         nv.check(L.tp_avgpool_nhwc_bf16(nv.ptr(cur), nv.ptr(xf), N, H * W, Cin, st), "tp_avgpool_nhwc_bf16")
         nv.mark("hmr_pool")
         return xf
+
+    @nv.device_guard
+    def features_from_frames(self, frames, crops):
+        """frames uint8 [F,H,W,3] RGB (CUDA), crops: the crop table (make_crop_table) -> [N,2048] fp32.  The device version of the
+        demo's crop + feature extraction (demo.py:183-198, lib/data_utils/_img_utils.py: get_single_image_crop_demo): each box is
+        cropped to 224x224 and normalised by tp_crop_normalize_bf16, bit-identical to the reference's cv2 / torchvision crop
+        rounded to bf16, then runs features_nhwc4."""
+        nv.require_cuda(frames, "frames")
+        if frames.dim() != 4 or frames.shape[3] != 3 or frames.dtype != torch.uint8:
+            raise ValueError(f"HMR.features_from_frames expects uint8 [F,H,W,3] frames, got {tuple(frames.shape)} {frames.dtype}")
+        crops = make_crop_table(crops, frames.device)
+        frames = frames.contiguous()
+        F, H, W, _ = frames.shape
+        N = crops.shape[0]
+        x4 = torch.empty(N, CROP, CROP, 4, device=frames.device, dtype=torch.bfloat16)
+        nv.check(nv.lib().tp_crop_normalize_bf16(nv.ptr(frames), F, H, W, nv.ptr(crops), N, nv.ptr(x4), nv.stream()),
+                 "tp_crop_normalize_bf16")
+        return self.features_nhwc4(x4)
 
     @nv.device_guard
     def forward(self, x, init_pose=None, init_shape=None, init_cam=None, n_iter=3, return_features=False):

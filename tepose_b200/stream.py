@@ -37,6 +37,7 @@ class WindowedTePose:
         self.use_graph = use_graph
         self._graph = None
         self._out = None
+        self.launches_per_replay = None
         self.seeded = False
 
     # ------------------------------------------------------------------ theta ring
@@ -89,20 +90,41 @@ class WindowedTePose:
         if not self.use_graph:
             return self._body()
         if self._graph is None:
-            keep = self.x.clone()
-            side = torch.cuda.Stream(device=self.device)
-            side.wait_stream(torch.cuda.current_stream(self.device))
-            with torch.cuda.stream(side):
-                self._body()                                     # packs weights, sets kernel attributes
-            torch.cuda.current_stream(self.device).wait_stream(side)
-            torch.cuda.synchronize(self.device)
-            self.x.copy_(keep)
-            self._graph = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(self._graph):
-                self._out = self._body()
-            self.x.copy_(keep)
+            self._graph, self._out, self.launches_per_replay = self._capture(self._body)
         self._graph.replay()
         return self._out
+
+    def _capture(self, fn):
+        """fn (which advances the rings in self.x) as a CUDA graph: one warm-up run on a side stream (packs weights, sets kernel
+        attributes), then the capture; the window is restored after each.  Returns (graph, fn's static output, native kernel
+        launches per replay)."""
+        keep = self.x.clone()
+        side = torch.cuda.Stream(device=self.device)
+        side.wait_stream(torch.cuda.current_stream(self.device))
+        with torch.cuda.stream(side):
+            fn()
+        torch.cuda.current_stream(self.device).wait_stream(side)
+        torch.cuda.synchronize(self.device)
+        self.x.copy_(keep)
+        graph = torch.cuda.CUDAGraph()
+        before = nv.lib().tp_launch_count()
+        with torch.cuda.graph(graph):
+            out = fn()
+        launches = int(nv.lib().tp_launch_count() - before)
+        self.x.copy_(keep)
+        return graph, out, launches
+
+    # ------------------------------------------------------------------ feature ring (tepose_b200.video)
+    @property
+    def features(self):
+        """[B,T,2048] view: the static features of the window, oldest frame first."""
+        return self.x[:, :, :FEAT]
+
+    def push_features(self, feats: torch.Tensor):
+        """Shift the feature ring by one frame: feats [B,2048] (on the device) becomes the newest frame of the window."""
+        f = self.features
+        f[:, :self.T - 1].copy_(f[:, 1:].clone())
+        f[:, self.T - 1].copy_(feats)
 
     # ------------------------------------------------------------------ whole sequence
     @torch.no_grad()
