@@ -311,7 +311,8 @@ class TemporalEncoder(nn.Module, GruKernels):
             hF0, hB0 = (None, None) if h0 is None else h0
             w, b, wu = d["w_hh"], d["b_hh"], d["w_um"]
             k2_prec = None
-            if last and "w_hh3" in d and h0 is None and B <= 32 and H // 16 <= 148 and "TP_FP32TC_NO_K2" not in os.environ:
+            # T == 1: every job is a single step from zero (gate math, no recurrent matmul), which BF16X3 does not take
+            if last and "w_hh3" in d and h0 is None and T > 1 and B <= 32 and H // 16 <= 148 and "TP_FP32TC_NO_K2" not in os.environ:
                 w = [d["w_hh3"][0], d["w_hh3"][1], w[2]]           # the single-step direction has no recurrent matmul
                 k2_prec = nv.PRECISION_BF16X3
             if last:

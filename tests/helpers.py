@@ -1,6 +1,8 @@
 """Shared test helpers: synthetic base_data directory, model construction, golden files, comparisons."""
 import ast
+import collections
 import contextlib
+import math
 import os
 import tempfile
 
@@ -10,6 +12,8 @@ import torch
 from oracle import synth, torch_ref
 
 FORWARD_OUTPUTS = ("theta", "verts", "kp_2d", "kp_3d", "rotmat")
+TC_BM = 128                                # k_gemm_bf16_tc tile rows
+U_OUT = {torch.bfloat16: 2.0 ** -8, torch.float32: 2.0 ** -24}
 
 
 @contextlib.contextmanager
@@ -77,3 +81,53 @@ def compare_outputs(got, ref, vert_tol=1e-4, rot_tol=1e-5, kp2d_tol=1e-3, label=
     assert errs["theta_cam_shape"] <= rot_tol * 10, (label, errs)
     assert errs["theta_pose_as_R"] <= rot_tol * 10, (label, errs)
     return errs
+
+
+GemmCheck = collections.namedtuple("GemmCheck", "ratio row col nans")
+
+
+def gemm_check(A, W, bias, residual, relu, out, max_bytes=2 << 30):
+    """out [rows, Cout] (bf16 or fp32, may be a strided window) against ref = act(A . W^T + bias + residual) in float64 from the
+    exact bf16 operands A [rows, KP], W [Cout, KP] (bias fp32 [Cout] or None, residual bf16 [rows, Cout] or None).
+
+    Bound per element: |out - ref| <= u |ref| + KP 2^-23 S,  S = |A| |W|^T + |bias| + |residual|.  u is one rounding of the
+    output (2^-8 bf16, 2^-24 fp32); the second term covers fp32 accumulation of the KP exact products and the two epilogue adds.
+    ReLU is 1-Lipschitz, so the bound holds after it.  Runs on the inputs' device, chunked over rows so that the float64
+    temporaries stay around `max_bytes`.  Returns the worst |out - ref| / bound, where it is, and the NaN count of `out`."""
+    rows, kp = A.shape
+    cout = W.shape[0]
+    assert W.shape[1] == kp and tuple(out.shape) == (rows, cout), (A.shape, W.shape, out.shape)
+    u, acc = U_OUT[out.dtype], kp * 2.0 ** -23
+    w = W.double()
+    wa = w.abs()
+    b = bias.double() if bias is not None else None
+    per_row = 8 * (2 * kp + 8 * cout)
+    chunk = max(TC_BM, (max_bytes - 16 * cout * kp) // per_row)
+    worst, where, nans = 0.0, (0, 0), 0
+    for r0 in range(0, rows, chunk):
+        a = A[r0:r0 + chunk].double()
+        ref, s = a @ w.T, a.abs() @ wa.T
+        del a
+        if b is not None:
+            ref += b
+            s += b.abs()
+        if residual is not None:
+            r = residual[r0:r0 + chunk].double()
+            ref += r
+            s += r.abs()
+            del r
+        if relu:
+            ref.clamp_(min=0.0)
+        bound = ref.abs().mul_(u).add_(s, alpha=acc)
+        del s
+        o = out[r0:r0 + chunk].double()
+        nan = torch.isnan(o)
+        nans += int(nan.sum())
+        err = (o - ref).abs_()
+        del o, ref
+        ratio = torch.where(err == 0, torch.zeros_like(err), err / bound)        # 0 / 0 -> 0, x / 0 -> inf
+        ratio.masked_fill_(nan | torch.isnan(ratio), math.inf)
+        i = int(ratio.argmax())
+        if float(ratio.view(-1)[i]) > worst or r0 == 0:
+            worst, where = float(ratio.view(-1)[i]), (r0 + i // cout, i % cout)
+    return GemmCheck(worst, where[0], where[1], nans)
