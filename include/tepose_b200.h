@@ -154,9 +154,15 @@ TP_API int tp_skinny_bf16_ex(const float* A, int64_t lda, const void* A_bf16, in
  * [n_start, n_start+n_cols) of W;  out[(m-m_start)*ldc + (n-n_start)] = dot + bias[n-n_start].
  * Epilogue options (flags; 0 = the plain fp32 output above): TP_GEMM_RELU clamps at zero, TP_GEMM_OUT_BF16 makes `out` a bf16
  * matrix (ldc in elements, ldc % 8 == 0), and a non-NULL `residual` (bf16 [m_rows, ldr], ldr % 8 == 0) is added before the clamp
- * -- the conv + folded BatchNorm (+ shortcut) + ReLU of a ResNet bottleneck (lib/models/spin.py:35-54) as one GEMM.          */
+ * -- the conv + folded BatchNorm (+ shortcut) + ReLU of a ResNet bottleneck (lib/models/spin.py:35-54) as one GEMM.
+ * Split layout (fp32-grade activations on bf16 operands): a row of C values v is stored as bf16 [hi(C) | lo(C) | hi(C)] with
+ * hi = RN_bf16(v), lo = RN_bf16(v - hi).  TP_GEMM_OUT_SPLIT3 writes the fp32 result v (after bias, residual and ReLU) that way:
+ * `out` is bf16, hi at column c, lo at n_cols + c, hi at 2 n_cols + c (ldc % 8 == 0, ldc >= 3 n_cols; TP_GEMM_OUT_BF16 is then
+ * ignored).  TP_GEMM_RES_SPLIT3: the residual rows are in split layout (ldr >= 3 n_cols) and hi + lo is added.              */
 #define TP_GEMM_RELU 1
 #define TP_GEMM_OUT_BF16 2
+#define TP_GEMM_OUT_SPLIT3 4
+#define TP_GEMM_RES_SPLIT3 8
 typedef struct tp_gemm_seg {
   int32_t m_start, m_rows;
   int32_t n_start, n_cols; /* n_cols % 16 == 0 */
@@ -188,6 +194,15 @@ TP_API int tp_im2col_nhwc_bf16(const void* in, void* out, int N, int H, int W, i
 TP_API int tp_maxpool3x3s2_nhwc_bf16(const void* in, void* out, int N, int H, int W, int C, void* stream);
 /* mean over the HW positions of [N, HW, C] bf16 -> [N, C] fp32 (nn.AvgPool2d(7) on the 7x7 map + view, spin.py:75,139-140) */
 TP_API int tp_avgpool_nhwc_bf16(const void* in, float* out, int N, int HW, int C, void* stream);
+/* Split-layout counterparts (precision "fp32_tc": every activation of C channels is bf16 [N,H,W,3C], [hi | lo | hi] per pixel as
+ * TP_GEMM_OUT_SPLIT3 writes it; tp_im2col_nhwc_bf16 gathers it unchanged with C' = 3C).
+ * x [N,C,H,W] fp32 -> y [N,H,W,3 CP] bf16, channels C..CP-1 of each block zero (CP = 4 for the RGB stem: 12 channels) */
+TP_API int tp_nchw_to_nhwc_split3(const float* x, void* y, int N, int C, int H, int W, int CP, void* stream);
+/* nn.MaxPool2d(3, 2, 1) on [N,H,W,3C] split rows: compares the represented values hi + lo exactly and writes the winning
+ * (hi, lo) pair (the first in (ky, kx) order on a tie); C % 8 == 0 */
+TP_API int tp_maxpool3x3s2_nhwc_split3(const void* in, void* out, int N, int H, int W, int C, void* stream);
+/* mean over the HW positions of hi + lo of [N, HW, 3C] split rows -> [N, C] fp32 (sequential fp32 sum, one division) */
+TP_API int tp_avgpool_nhwc_split3(const void* in, float* out, int N, int HW, int C, void* stream);
 
 /* ------------------------------------------------------------------ demo front end: person crops on the device
  * One row of the crop table: the box of a tracked person (lib/data_utils/_img_utils.py: get_single_image_crop_demo, bbox =
@@ -208,6 +223,11 @@ typedef struct tp_crop {
  * 1/1024 pixel).  crops 4-byte, out 16-byte aligned. */
 TP_API int tp_crop_normalize_bf16(const void* frames, int F, int H, int W, const tp_crop* crops, int N, void* out,
                                   void* stream);
+/* The same crop and the same fp32 normalisation, written in split layout instead of rounded: out [N,224,224,12] bf16,
+ * [hi(4) | lo(4) | hi(4)] per pixel with channel 3 of each block zero (the stem input of precision "fp32_tc").  Same argument
+ * checks and the same behaviour for a bad frame index under capture. */
+TP_API int tp_crop_normalize_split3(const void* frames, int F, int H, int W, const tp_crop* crops, int N, void* out,
+                                    void* stream);
 
 /* ------------------------------------------------------------------ GRU recurrence (K2)
  * One direction of one torch.nn.GRU layer (lib/models/tepose.py:53-64,73,76) given the

@@ -3,10 +3,11 @@
 - push latency at B = 1 for a 1920x1080 RGB frame: host clock around push() + synchronize, p50 / p99 over --pushes frames,
   with the frame in pinned host memory (it is uploaded inside the push) and already on the device;
 - frames per second at B = 32 (32 people per frame): back-to-back pushes, one synchronize at the end;
-- tp_crop_normalize_bf16 alone at N = 32 crops: CUDA events around a graph of 20 launches, and the bytes it writes.
+- the crop kernel alone at N = 32 crops: CUDA events around a graph of 20 launches, and the bytes it writes.
 
-The model is the released configuration (TePose T16 L1 H2048 bf16, VIBE L2 H1024 bootstrap) with synthetic weights; the
-card's name and power limit are read in the same run.
+--precision bf16 (default): the released configuration (HMR and TePose T16 L1 H2048 bf16, VIBE L2 H1024 bootstrap) with
+synthetic weights.  --precision fp32_tc: HMR and TePose in "fp32_tc" (split-bf16 tensor-core operands, fp32-grade results;
+tp_crop_normalize_split3), VIBE in fp32.  The card's name and power limit are read in the same run.
 """
 import argparse
 import json
@@ -65,16 +66,20 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--pushes", type=int, default=300)
     ap.add_argument("--clip", type=int, default=8, help="distinct frames cycled through")
+    ap.add_argument("--precision", choices=["bf16", "fp32_tc"], default="bf16")
     args = ap.parse_args()
     torch.cuda.init()
     dev = "cuda:0"
-    hmr = build_synthetic_hmr(0, dev)
-    model, _ = build_synthetic_model(0, T, 1, 2048, "bf16", dev)
-    vibe, _ = build_synthetic_vibe(0, T, 2, 1024, True, False, True, "bf16", dev)
+    split = args.precision == "fp32_tc"
+    hmr = build_synthetic_hmr(0, dev, precision=args.precision)
+    model, _ = build_synthetic_model(0, T, 1, 2048, args.precision, dev)
+    vibe, _ = build_synthetic_vibe(0, T, 2, 1024, True, False, True, "fp32" if split else "bf16", dev)
     host = torch.from_numpy(crop_ref.sample_frames(1, args.clip, H, W)).pin_memory()
     frames_host = [host[i:i + 1] for i in range(args.clip)]
     frames_dev = [f.to(dev) for f in frames_host]
-    res = {"card": card(), "frame": [H, W], "model": "TePose T16 L1 H2048 bf16, VIBE L2 H1024 bf16, synthetic weights"}
+    res = {"card": card(), "frame": [H, W], "precision": args.precision,
+           "model": (f"HMR {args.precision}, TePose T16 L1 H2048 {args.precision}, VIBE L2 H1024 {'fp32' if split else 'bf16'}, "
+                     "synthetic weights")}
 
     for where, frames in (("pinned_host", frames_host), ("device", frames_dev)):
         vt = VideoTePose(hmr, model, vibe, batch=1)
@@ -94,11 +99,12 @@ def main():
     # the crop kernel alone, N = 32, inside a graph (eager calls read the table back to check frame indices)
     N, reps = 32, 20
     table = make_crop_table(boxes(N, 0), dev)
-    out = torch.empty(N, 224, 224, 4, dtype=torch.bfloat16, device=dev)
+    out = torch.empty(N, 224, 224, hmr.stem_channels, dtype=torch.bfloat16, device=dev)
     fr = frames_dev[0]
+    crop = nv.lib().tp_crop_normalize_split3 if split else nv.lib().tp_crop_normalize_bf16
 
     def launch():
-        nv.check(nv.lib().tp_crop_normalize_bf16(nv.ptr(fr), 1, H, W, nv.ptr(table), N, nv.ptr(out), nv.stream()))
+        nv.check(crop(nv.ptr(fr), 1, H, W, nv.ptr(table), N, nv.ptr(out), nv.stream()))
     launch()
     torch.cuda.synchronize()
     g = torch.cuda.CUDAGraph()

@@ -18,7 +18,7 @@ LIB_PATH = os.environ.get("TEPOSE_B200_LIB") or os.path.join(_HERE, "libtepose_b
 PRECISION_FP32, PRECISION_BF16, PRECISION_BF16X3 = 0, 1, 2
 POSE_ROTMAT, POSE_AXIS_ANGLE, POSE_ROT6D = 0, 1, 2
 RODRIGUES_SMPLX, RODRIGUES_QUAT = 0, 1
-GEMM_RELU, GEMM_OUT_BF16 = 1, 2            # tp_gemm_seg.flags
+GEMM_RELU, GEMM_OUT_BF16, GEMM_OUT_SPLIT3, GEMM_RES_SPLIT3 = 1, 2, 4, 8      # tp_gemm_seg.flags
 # "fp32_tc": fp32-grade results with the two big contractions (K1 input projection, K2 recurrence) on tensor cores as 3-term bf16
 # splits (TP_PRECISION_BF16X3); every other stage runs exactly as in "fp32", which is the code the C ABI sees for them
 PRECISIONS = {"fp32": PRECISION_FP32, "bf16": PRECISION_BF16, "fp32_tc": PRECISION_FP32}
@@ -38,6 +38,7 @@ EXPORTS = [
     "tp_tepose_loss_workspace_bytes", "tp_tepose_loss",
     "tp_nchw_to_nhwc_bf16", "tp_im2col_nhwc_bf16", "tp_maxpool3x3s2_nhwc_bf16", "tp_avgpool_nhwc_bf16",
     "tp_crop_normalize_bf16",
+    "tp_nchw_to_nhwc_split3", "tp_maxpool3x3s2_nhwc_split3", "tp_avgpool_nhwc_split3", "tp_crop_normalize_split3",
 ]
 
 vp, i32, i64, f32, sz = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
@@ -84,6 +85,10 @@ _SIGNATURES = {
     "tp_maxpool3x3s2_nhwc_bf16": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
     "tp_avgpool_nhwc_bf16": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, vp]),
     "tp_crop_normalize_bf16": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, vp, C.c_int, vp, vp]),
+    "tp_nchw_to_nhwc_split3": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
+    "tp_maxpool3x3s2_nhwc_split3": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
+    "tp_avgpool_nhwc_split3": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, vp]),
+    "tp_crop_normalize_split3": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, vp, C.c_int, vp, vp]),
     "tp_device_info": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(sz)]),
     "tp_rot6d_to_rotmat": (C.c_int, [vp, vp, i64, vp]),
     "tp_rotmat_to_angle_axis": (C.c_int, [vp, vp, i64, vp]),

@@ -6,13 +6,24 @@
 
 namespace tp {
 
-// x [N,C,H,W] fp32 -> y [N,H,W,CP] bf16 (channels c >= C are zero); CP = 4 for the RGB stem
+// x [N,C,H,W] fp32 -> y [N,H,W,CP] bf16 (channels c >= C are zero); CP = 4 for the RGB stem.
+// SPLIT: y [N,H,W,3 CP], [hi | lo | hi] per pixel, hi = RN_bf16(v), lo = RN_bf16(v - hi).
+template <bool SPLIT>
 __global__ void k_nchw_to_nhwc(const float* __restrict__ x, __nv_bfloat16* __restrict__ y, int N, int C, int H, int W, int CP) {
   const int64_t total = (int64_t)N * H * W;
   for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
     const int64_t n = i / ((int64_t)H * W), hw = i - n * H * W;
-    for (int c = 0; c < CP; ++c)
-      y[i * CP + c] = __float2bfloat16_rn(c < C ? x[(n * C + c) * (int64_t)H * W + hw] : 0.0f);
+    for (int c = 0; c < CP; ++c) {
+      const float v = c < C ? x[(n * C + c) * (int64_t)H * W + hw] : 0.0f;
+      const __nv_bfloat16 hi = __float2bfloat16_rn(v);
+      if (SPLIT) {
+        y[i * 3 * CP + c] = hi;
+        y[i * 3 * CP + CP + c] = __float2bfloat16_rn(v - __bfloat162float(hi));
+        y[i * 3 * CP + 2 * CP + c] = hi;
+      } else {
+        y[i * CP + c] = hi;
+      }
+    }
   }
 }
 
@@ -89,6 +100,57 @@ __global__ void k_avgpool(const __nv_bfloat16* __restrict__ in, float* __restric
   }
 }
 
+// MaxPool2d(3, 2, 1) on split rows [N,H,W,3C]: the represented value hi + lo is exact in fp64; strict '>' keeps the first
+// maximum in (ky, kx) order.  8 channels per thread.
+__global__ void k_maxpool3x3s2_split3(const __nv_bfloat16* __restrict__ in, __nv_bfloat16* __restrict__ out, int N, int H, int W, int C,
+                                      int Ho, int Wo) {
+  const int cv = C / 8;
+  const int64_t total = (int64_t)N * Ho * Wo * cv;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int c = (int)(i % cv) * 8;
+    const int64_t pix = i / cv;
+    const int wo = (int)(pix % Wo), ho = (int)((pix / Wo) % Ho), n = (int)(pix / ((int64_t)Wo * Ho));
+    double m[8];
+    __align__(16) __nv_bfloat16 bh[8], bl[8];
+#pragma unroll
+    for (int u = 0; u < 8; ++u) { m[u] = -INFINITY; bh[u] = __float2bfloat16_rn(-INFINITY); bl[u] = __float2bfloat16_rn(0.0f); }
+    for (int ky = 0; ky < 3; ++ky)
+      for (int kx = 0; kx < 3; ++kx) {
+        const int hi = ho * 2 - 1 + ky, wi = wo * 2 - 1 + kx;
+        if (hi < 0 || hi >= H || wi < 0 || wi >= W) continue;
+        const __nv_bfloat16* src = in + (((int64_t)n * H + hi) * W + wi) * 3 * C + c;
+        __align__(16) __nv_bfloat16 h[8], l[8];
+        *reinterpret_cast<uint4*>(h) = *reinterpret_cast<const uint4*>(src);
+        *reinterpret_cast<uint4*>(l) = *reinterpret_cast<const uint4*>(src + C);
+#pragma unroll
+        for (int u = 0; u < 8; ++u) {
+          const double v = (double)__bfloat162float(h[u]) + (double)__bfloat162float(l[u]);
+          if (v > m[u]) { m[u] = v; bh[u] = h[u]; bl[u] = l[u]; }
+        }
+      }
+    __nv_bfloat16* dst = out + pix * 3 * C + c;
+    *reinterpret_cast<uint4*>(dst) = *reinterpret_cast<const uint4*>(bh);
+    *reinterpret_cast<uint4*>(dst + C) = *reinterpret_cast<const uint4*>(bl);
+    *reinterpret_cast<uint4*>(dst + 2 * C) = *reinterpret_cast<const uint4*>(bh);
+  }
+}
+
+// mean of hi + lo over HW positions of split rows [N,HW,3C] -> [N,C] fp32 (hi + lo is exact in fp32 for a split the GEMM
+// epilogue wrote)
+__global__ void k_avgpool_split3(const __nv_bfloat16* __restrict__ in, float* __restrict__ out, int N, int HW, int C) {
+  const int64_t total = (int64_t)N * C;
+  for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < total; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t n = i / C;
+    const int c = (int)(i - n * C);
+    float s = 0.0f;
+    for (int p = 0; p < HW; ++p) {
+      const __nv_bfloat16* r = in + (n * HW + p) * 3 * C + c;
+      s += __bfloat162float(r[0]) + __bfloat162float(r[C]);
+    }
+    out[i] = s / (float)HW;
+  }
+}
+
 static unsigned grid_for(int64_t total) {
   int64_t g = (total + 255) / 256;
   const int64_t cap = (int64_t)sm_count() * 16;
@@ -101,7 +163,31 @@ using namespace tp;
 
 extern "C" int tp_nchw_to_nhwc_bf16(const float* x, void* y, int N, int C, int H, int W, int CP, void* stream) {
   TP_CHECK_ARG(x && y && N > 0 && C > 0 && H > 0 && W > 0 && CP >= C, "tp_nchw_to_nhwc_bf16: bad arguments");
-  k_nchw_to_nhwc<<<grid_for((int64_t)N * H * W), 256, 0, (cudaStream_t)stream>>>(x, reinterpret_cast<__nv_bfloat16*>(y), N, C, H, W, CP);
+  k_nchw_to_nhwc<false><<<grid_for((int64_t)N * H * W), 256, 0, (cudaStream_t)stream>>>(x, reinterpret_cast<__nv_bfloat16*>(y), N, C, H, W, CP);
+  TP_LAUNCH_CHECK();
+  return TP_OK;
+}
+
+extern "C" int tp_nchw_to_nhwc_split3(const float* x, void* y, int N, int C, int H, int W, int CP, void* stream) {
+  TP_CHECK_ARG(x && y && N > 0 && C > 0 && H > 0 && W > 0 && CP >= C, "tp_nchw_to_nhwc_split3: bad arguments");
+  k_nchw_to_nhwc<true><<<grid_for((int64_t)N * H * W), 256, 0, (cudaStream_t)stream>>>(x, reinterpret_cast<__nv_bfloat16*>(y), N, C, H, W, CP);
+  TP_LAUNCH_CHECK();
+  return TP_OK;
+}
+
+extern "C" int tp_maxpool3x3s2_nhwc_split3(const void* in, void* out, int N, int H, int W, int C, void* stream) {
+  TP_CHECK_ARG(in && out && N > 0 && H > 0 && W > 0 && C > 0 && C % 8 == 0, "tp_maxpool3x3s2_nhwc_split3: bad arguments (C %% 8 == 0)");
+  TP_CHECK_ARG(aligned16(in) && aligned16(out), "tp_maxpool3x3s2_nhwc_split3: pointers must be 16-byte aligned");
+  const int Ho = (H + 2 - 3) / 2 + 1, Wo = (W + 2 - 3) / 2 + 1;
+  k_maxpool3x3s2_split3<<<grid_for((int64_t)N * Ho * Wo * (C / 8)), 256, 0, (cudaStream_t)stream>>>(
+      reinterpret_cast<const __nv_bfloat16*>(in), reinterpret_cast<__nv_bfloat16*>(out), N, H, W, C, Ho, Wo);
+  TP_LAUNCH_CHECK();
+  return TP_OK;
+}
+
+extern "C" int tp_avgpool_nhwc_split3(const void* in, float* out, int N, int HW, int C, void* stream) {
+  TP_CHECK_ARG(in && out && N > 0 && HW > 0 && C > 0, "tp_avgpool_nhwc_split3: bad arguments");
+  k_avgpool_split3<<<grid_for((int64_t)N * C), 256, 0, (cudaStream_t)stream>>>(reinterpret_cast<const __nv_bfloat16*>(in), out, N, HW, C);
   TP_LAUNCH_CHECK();
   return TP_OK;
 }

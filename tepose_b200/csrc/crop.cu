@@ -93,17 +93,20 @@ __device__ __forceinline__ void crop_inverse_map(const tp_crop& c, double iM[6])
 }
 
 // grid (blocks per crop, N); every block covers the pairs p = blockIdx.x * kThreads + threadIdx.x (+ gridDim.x * kThreads) of
-// its crop.  out [N,224,224,4] bf16; channel 3 is zero.
+// its crop.  out [N,224,224,4] bf16, channel 3 zero; SPLIT: out [N,224,224,12] bf16, [hi(4) | lo(4) | hi(4)] per pixel of the
+// fp32 normalised value (hi = RN_bf16(v), lo = RN_bf16(v - hi)), channel 3 of each block zero.
+template <bool SPLIT>
 __global__ void __launch_bounds__(kThreads) k_crop_normalize(const uint8_t* __restrict__ frames, int F, int H, int W,
                                                              const tp_crop* __restrict__ crops, __nv_bfloat16* __restrict__ out) {
+  constexpr int CH = SPLIT ? 12 : 4;                     // output channels per pixel
   __shared__ double s_map[6];
-  __shared__ __nv_bfloat16 s_lut[3][256];                // byte value -> normalized bf16, per channel
+  __shared__ float s_lut[3][256];                        // byte value -> normalized fp32, per channel
   __shared__ int s_frame;
   const int n = blockIdx.y;
   for (int i = threadIdx.x; i < 3 * 256; i += kThreads) {
     const int ch = i >> 8;
     const float mean = ch == 0 ? 0.485f : (ch == 1 ? 0.456f : 0.406f), stdv = ch == 0 ? 0.229f : (ch == 1 ? 0.224f : 0.225f);
-    s_lut[ch][i & 255] = __float2bfloat16_rn(__fdiv_rn(__fsub_rn(__fdiv_rn((float)(i & 255), 255.0f), mean), stdv));
+    s_lut[ch][i & 255] = __fdiv_rn(__fsub_rn(__fdiv_rn((float)(i & 255), 255.0f), mean), stdv);
   }
   if (threadIdx.x < 32) {
     const tp_crop c = crops[n];
@@ -120,13 +123,13 @@ __global__ void __launch_bounds__(kThreads) k_crop_normalize(const uint8_t* __re
   const double m0 = s_map[0], m1 = s_map[1], m2 = s_map[2], m3 = s_map[3], m4 = s_map[4], m5 = s_map[5];
   const int f = s_frame;
   const uint8_t* img = frames + (size_t)(f < 0 ? 0 : f) * H * W * 3;
-  uint4* dst = reinterpret_cast<uint4*>(out + (size_t)n * kCrop * kCrop * 4);
+  uint4* dst = reinterpret_cast<uint4*>(out + (size_t)n * kCrop * kCrop * CH);
   for (int p = blockIdx.x * kThreads + threadIdx.x; p < kPairs; p += gridDim.x * kThreads) {
     const int y = p / kPairsPerRow, x0 = (p - y * kPairsPerRow) * 2;
-    __align__(16) __nv_bfloat16 o[8];
+    __align__(16) __nv_bfloat16 o[2 * CH];
     if (f < 0) {
 #pragma unroll
-      for (int u = 0; u < 8; ++u) o[u] = __float2bfloat16_rn(0.0f);
+      for (int u = 0; u < 2 * CH; ++u) o[u] = __float2bfloat16_rn(0.0f);
     } else {
       // cv2 WarpAffineInvoker: X0, Y0 per row (+ 16: half of a 1/32 step), adelta / bdelta per column, in 1/1024 pixel
       const int X0 = __double2int_rn(dmul(dadd(dmul(m1, (double)y), m2), 1024.0)) + 16;
@@ -155,25 +158,30 @@ __global__ void __launch_bounds__(kThreads) k_crop_normalize(const uint8_t* __re
           }
         }
 #pragma unroll
-        for (int ch = 0; ch < 3; ++ch) o[4 * u + ch] = s_lut[ch][(acc[ch] + (1 << 14)) >> 15];
-        o[4 * u + 3] = __float2bfloat16_rn(0.0f);
+        for (int ch = 0; ch < 4; ++ch) {
+          const float v = ch < 3 ? s_lut[ch][(acc[ch] + (1 << 14)) >> 15] : 0.0f;
+          const __nv_bfloat16 hi = __float2bfloat16_rn(v);
+          o[CH * u + ch] = hi;
+          if (SPLIT) {
+            o[CH * u + 4 + ch] = __float2bfloat16_rn(v - __bfloat162float(hi));
+            o[CH * u + 8 + ch] = hi;
+          }
+        }
       }
     }
-    dst[p] = *reinterpret_cast<const uint4*>(o);
+#pragma unroll
+    for (int k = 0; k < CH / 4; ++k) dst[p * (CH / 4) + k] = reinterpret_cast<const uint4*>(o)[k];
   }
 }
 
-}  // namespace tp
-
-using namespace tp;
-
-extern "C" int tp_crop_normalize_bf16(const void* frames, int F, int H, int W, const tp_crop* crops, int N, void* out,
-                                      void* stream) {
-  TP_CHECK_ARG(frames && crops && out, "tp_crop_normalize_bf16: null pointer");
+template <bool SPLIT>
+static int crop_normalize(const char* name, const void* frames, int F, int H, int W, const tp_crop* crops, int N, void* out,
+                          void* stream) {
+  TP_CHECK_ARG(frames && crops && out, "%s: null pointer", name);
   TP_CHECK_ARG(F > 0 && H > 0 && W > 0 && N > 0 && N <= 65535,
-               "tp_crop_normalize_bf16: need F, H, W > 0 and 0 < N <= 65535 (F=%d H=%d W=%d N=%d)", F, H, W, N);
+               "%s: need F, H, W > 0 and 0 < N <= 65535 (F=%d H=%d W=%d N=%d)", name, F, H, W, N);
   TP_CHECK_ARG((reinterpret_cast<uintptr_t>(crops) & 3u) == 0 && aligned16(out),
-               "tp_crop_normalize_bf16: crops must be 4-byte and out 16-byte aligned");
+               "%s: crops must be 4-byte and out 16-byte aligned", name);
   cudaStream_t st = (cudaStream_t)stream;
   cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
   TP_CUDA(cudaStreamIsCapturing(st, &cap));
@@ -182,13 +190,26 @@ extern "C" int tp_crop_normalize_bf16(const void* frames, int F, int H, int W, c
     TP_CUDA(cudaMemcpyAsync(host.data(), crops, (size_t)N * sizeof(tp_crop), cudaMemcpyDefault, st));
     TP_CUDA(cudaStreamSynchronize(st));
     for (int i = 0; i < N; ++i)
-      TP_CHECK_ARG(host[i].frame >= 0 && host[i].frame < F, "tp_crop_normalize_bf16: crop %d names frame %d of %d", i,
-                   host[i].frame, F);
+      TP_CHECK_ARG(host[i].frame >= 0 && host[i].frame < F, "%s: crop %d names frame %d of %d", name, i, host[i].frame, F);
   }
   const int per_crop = (int)ceil_div(kPairs, kThreads);
   const int bx = (int)std::min<int64_t>(per_crop, std::max<int64_t>(1, ceil_div((int64_t)sm_count() * 8, N)));
-  k_crop_normalize<<<dim3(bx, N), kThreads, 0, st>>>(reinterpret_cast<const uint8_t*>(frames), F, H, W, crops,
-                                                      reinterpret_cast<__nv_bfloat16*>(out));
+  k_crop_normalize<SPLIT><<<dim3(bx, N), kThreads, 0, st>>>(reinterpret_cast<const uint8_t*>(frames), F, H, W, crops,
+                                                             reinterpret_cast<__nv_bfloat16*>(out));
   TP_LAUNCH_CHECK();
   return TP_OK;
+}
+
+}  // namespace tp
+
+using namespace tp;
+
+extern "C" int tp_crop_normalize_bf16(const void* frames, int F, int H, int W, const tp_crop* crops, int N, void* out,
+                                      void* stream) {
+  return crop_normalize<false>("tp_crop_normalize_bf16", frames, F, H, W, crops, N, out, stream);
+}
+
+extern "C" int tp_crop_normalize_split3(const void* frames, int F, int H, int W, const tp_crop* crops, int N, void* out,
+                                        void* stream) {
+  return crop_normalize<true>("tp_crop_normalize_split3", frames, F, H, W, crops, N, out, stream);
 }

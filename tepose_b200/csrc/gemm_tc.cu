@@ -60,7 +60,47 @@ __device__ __forceinline__ TcTile tc_decode(const TcParams& p, int tile) {
   return t;
 }
 
-template <int BN>
+// TP_GEMM_RES_SPLIT3: r points at the hi block of 8 columns of a split-layout row [hi | lo | hi]; adds hi + lo, which is exact
+// in fp32 (lo carries the bits of the value below hi's 8).
+__device__ __forceinline__ void tc_add_res_split3(float o[8], const __nv_bfloat16* r, int n_cols, int n, bool full) {
+  if (full) {
+    const uint4 hv = *reinterpret_cast<const uint4*>(r), lv = *reinterpret_cast<const uint4*>(r + n_cols);
+    const __nv_bfloat162* h = reinterpret_cast<const __nv_bfloat162*>(&hv);
+    const __nv_bfloat162* l = reinterpret_cast<const __nv_bfloat162*>(&lv);
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      const float2 a = __bfloat1622float2(h[u]), b = __bfloat1622float2(l[u]);
+      o[2 * u] += a.x + b.x;
+      o[2 * u + 1] += a.y + b.y;
+    }
+  } else {
+    for (int u = 0; u < 8; ++u)
+      if (n + u < n_cols) o[u] += __bfloat162float(r[u]) + __bfloat162float(r[n_cols + u]);
+  }
+}
+
+// TP_GEMM_OUT_SPLIT3: v -> hi = RN_bf16(v) at column c, lo = RN_bf16(v - hi) at n_cols + c, hi again at 2 n_cols + c
+// (v - hi is exact in fp32).  d points at column c of the hi block.
+__device__ __forceinline__ void tc_store_split3(const float o[8], __nv_bfloat16* d, int n_cols, int n, bool full) {
+  __align__(16) __nv_bfloat16 hi[8], lo[8];
+#pragma unroll
+  for (int u = 0; u < 8; ++u) {
+    hi[u] = __float2bfloat16_rn(o[u]);
+    lo[u] = __float2bfloat16_rn(o[u] - __bfloat162float(hi[u]));
+  }
+  if (full) {
+    *reinterpret_cast<uint4*>(d) = *reinterpret_cast<const uint4*>(hi);
+    *reinterpret_cast<uint4*>(d + n_cols) = *reinterpret_cast<const uint4*>(lo);
+    *reinterpret_cast<uint4*>(d + 2 * n_cols) = *reinterpret_cast<const uint4*>(hi);
+  } else {
+    for (int u = 0; u < 8; ++u)
+      if (n + u < n_cols) { d[u] = hi[u]; d[n_cols + u] = lo[u]; d[2 * n_cols + u] = hi[u]; }
+  }
+}
+
+// SPLIT: the launch has a segment with TP_GEMM_OUT_SPLIT3 / TP_GEMM_RES_SPLIT3.  A compile-time switch: the split branches in
+// the epilogue loop cost the bf16 HMR convolutions 7 % when present at run time in every launch.
+template <int BN, bool SPLIT>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 k_gemm_bf16_tc(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_w, const TcParams p) {
   using Cfg = TcCfg<BN>;
@@ -154,6 +194,7 @@ k_gemm_bf16_tc(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
       const int row = t.m0 + lg * 32 + lane;             // segment-local output row of this thread (= its TMEM lane)
       const bool row_ok = row < t.sg.m_rows;
       const bool relu = (t.sg.flags & TP_GEMM_RELU) != 0, out_lp = (t.sg.flags & TP_GEMM_OUT_BF16) != 0;
+      const bool out_split = SPLIT && (t.sg.flags & TP_GEMM_OUT_SPLIT3) != 0, res_split = SPLIT && (t.sg.flags & TP_GEMM_RES_SPLIT3) != 0;
       const bool vec_ok = ((t.sg.ldc & 3) == 0) && ((reinterpret_cast<uintptr_t>(t.sg.out) & 15) == 0);
       float* orow = t.sg.out + (int64_t)row * t.sg.ldc + t.n0;
       __nv_bfloat16* orow_lp = reinterpret_cast<__nv_bfloat16*>(t.sg.out) + (int64_t)row * t.sg.ldc + t.n0;
@@ -172,7 +213,9 @@ k_gemm_bf16_tc(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 #pragma unroll
             for (int u = 0; u < 8; ++u) o[u] = __uint_as_float(v[q * 8 + u]) + s_bias[acc][c0 + q * 8 + u];
             const bool full = n + 7 < t.sg.n_cols;
-            if (rrow && full) {
+            if (rrow && res_split) {
+              tc_add_res_split3(o, rrow + c0 + q * 8, t.sg.n_cols, n, full);
+            } else if (rrow && full) {
               const uint4 rv = *reinterpret_cast<const uint4*>(rrow + c0 + q * 8);
               const __nv_bfloat162* rh = reinterpret_cast<const __nv_bfloat162*>(&rv);
 #pragma unroll
@@ -185,7 +228,9 @@ k_gemm_bf16_tc(const __grid_constant__ CUtensorMap map_a, const __grid_constant_
 #pragma unroll
               for (int u = 0; u < 8; ++u) o[u] = fmaxf(o[u], 0.0f);
             }
-            if (out_lp) {
+            if (out_split) {
+              tc_store_split3(o, orow_lp + c0 + q * 8, t.sg.n_cols, n, full);
+            } else if (out_lp) {
               if (full) {
                 __nv_bfloat162 h[4];
 #pragma unroll
@@ -380,6 +425,7 @@ k_gemm_bf16_tc2(const __grid_constant__ CUtensorMap map_a, const __grid_constant
       const int row = t.m0 + (int)rank * TC_BM + lg * 32 + lane;
       const bool row_ok = row < t.sg.m_rows;
       const bool relu = (t.sg.flags & TP_GEMM_RELU) != 0, out_lp = (t.sg.flags & TP_GEMM_OUT_BF16) != 0;
+      const bool out_split = (t.sg.flags & TP_GEMM_OUT_SPLIT3) != 0, res_split = (t.sg.flags & TP_GEMM_RES_SPLIT3) != 0;
       const bool vec_ok = ((t.sg.ldc & 3) == 0) && ((reinterpret_cast<uintptr_t>(t.sg.out) & 15) == 0);
       float* orow = t.sg.out + (int64_t)row * t.sg.ldc + t.n0;
       __nv_bfloat16* orow_lp = reinterpret_cast<__nv_bfloat16*>(t.sg.out) + (int64_t)row * t.sg.ldc + t.n0;
@@ -399,7 +445,9 @@ k_gemm_bf16_tc2(const __grid_constant__ CUtensorMap map_a, const __grid_constant
 #pragma unroll
             for (int u = 0; u < 8; ++u) o[u] = __uint_as_float(v[q * 8 + u]) + s_bias[acc][c0 + q * 8 + u];
             const bool full = n + 7 < t.sg.n_cols;
-            if (rrow) {
+            if (rrow && res_split) {
+              tc_add_res_split3(o, rrow + c0 + q * 8, t.sg.n_cols, n, full);
+            } else if (rrow) {
               for (int u = 0; u < 8; ++u)
                 if (n + u < t.sg.n_cols) o[u] += __bfloat162float(rrow[c0 + q * 8 + u]);
             }
@@ -407,7 +455,9 @@ k_gemm_bf16_tc2(const __grid_constant__ CUtensorMap map_a, const __grid_constant
 #pragma unroll
               for (int u = 0; u < 8; ++u) o[u] = fmaxf(o[u], 0.0f);
             }
-            if (out_lp) {
+            if (out_split) {
+              tc_store_split3(o, orow_lp + c0 + q * 8, t.sg.n_cols, n, full);
+            } else if (out_lp) {
               for (int u = 0; u < 8; ++u)
                 if (n + u < t.sg.n_cols) orow_lp[c0 + q * 8 + u] = __float2bfloat16_rn(o[u]);
             } else if (full && vec_ok) {
@@ -464,6 +514,16 @@ static int make_map(CUtensorMap* map, const void* base, int rows, int kp, int bo
   return TP_OK;
 }
 
+template <int BN, bool SPLIT>
+static int launch_tc(const CUtensorMap& map_a, const CUtensorMap& map_w, const TcParams& p, int grid, cudaStream_t stream) {
+  using Cfg = TcCfg<BN>;
+  const size_t smem = (size_t)Cfg::STAGES * Cfg::STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
+  TP_CUDA(cudaFuncSetAttribute(k_gemm_bf16_tc<BN, SPLIT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  PdlConfig lc(dim3((unsigned)grid), dim3(TC_THREADS), smem, stream);
+  TP_CUDA(cudaLaunchKernelEx(&lc.cfg, k_gemm_bf16_tc<BN, SPLIT>, map_a, map_w, p));
+  return TP_OK;
+}
+
 }  // namespace tp
 
 using namespace tp;
@@ -498,6 +558,10 @@ extern "C" int tp_gemm_bf16_tc(const void* A, int a_rows, const void* W, int w_r
     TP_CHECK_ARG(sg.n_cols % 16 == 0, "tp_gemm_bf16_tc: segment %d: n_cols=%d must be a multiple of 16", i, sg.n_cols);
     TP_CHECK_ARG(!(sg.flags & TP_GEMM_OUT_BF16) || (sg.ldc % 8 == 0 && aligned16(sg.out)), "tp_gemm_bf16_tc: segment %d: bf16 output needs ldc %% 8 == 0 and 16-byte alignment", i);
     TP_CHECK_ARG(!sg.residual || (sg.ldr % 8 == 0 && aligned16(sg.residual)), "tp_gemm_bf16_tc: segment %d: residual needs ldr %% 8 == 0 and 16-byte alignment", i);
+    TP_CHECK_ARG(!(sg.flags & TP_GEMM_OUT_SPLIT3) || (sg.ldc % 8 == 0 && sg.ldc >= 3 * (int64_t)sg.n_cols && aligned16(sg.out)),
+                 "tp_gemm_bf16_tc: segment %d: split output needs ldc %% 8 == 0, ldc >= 3 n_cols and 16-byte alignment", i);
+    TP_CHECK_ARG(!(sg.flags & TP_GEMM_RES_SPLIT3) || (sg.residual && sg.ldr >= 3 * sg.n_cols),
+                 "tp_gemm_bf16_tc: segment %d: split residual needs a residual with ldr >= 3 n_cols", i);
     p.seg[i] = sg;
     p.tile_begin[i] = tiles;
     tiles += (int)(ceil_div(sg.m_rows, TC_BM) * ceil_div(sg.n_cols, bn));
@@ -538,19 +602,12 @@ extern "C" int tp_gemm_bf16_tc(const void* A, int a_rows, const void* W, int w_r
     return TP_OK;
   }
   const int grid = tiles < sm_count() ? tiles : sm_count();      // persistent: CTA c takes tiles c, c + grid, ...
-  if (bn == 192) {
-    using Cfg = TcCfg<192>;
-    const size_t smem = (size_t)Cfg::STAGES * Cfg::STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
-    TP_CUDA(cudaFuncSetAttribute(k_gemm_bf16_tc<192>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    PdlConfig lc(dim3((unsigned)grid), dim3(TC_THREADS), smem, (cudaStream_t)stream);
-    TP_CUDA(cudaLaunchKernelEx(&lc.cfg, k_gemm_bf16_tc<192>, map_a, map_w, p));
-  } else {
-    using Cfg = TcCfg<128>;
-    const size_t smem = (size_t)Cfg::STAGES * Cfg::STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
-    TP_CUDA(cudaFuncSetAttribute(k_gemm_bf16_tc<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    PdlConfig lc(dim3((unsigned)grid), dim3(TC_THREADS), smem, (cudaStream_t)stream);
-    TP_CUDA(cudaLaunchKernelEx(&lc.cfg, k_gemm_bf16_tc<128>, map_a, map_w, p));
-  }
+  bool split = false;
+  for (int i = 0; i < nseg; ++i) split |= (segs[i].flags & (TP_GEMM_OUT_SPLIT3 | TP_GEMM_RES_SPLIT3)) != 0;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (bn == 192) rc = split ? launch_tc<192, true>(map_a, map_w, p, grid, st) : launch_tc<192, false>(map_a, map_w, p, grid, st);
+  else rc = split ? launch_tc<128, true>(map_a, map_w, p, grid, st) : launch_tc<128, false>(map_a, map_w, p, grid, st);
+  if (rc != TP_OK) return rc;
   TP_LAUNCH_CHECK();
   return TP_OK;
 }

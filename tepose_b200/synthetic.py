@@ -351,8 +351,8 @@ def make_image_batch(seed: int, n: int, size: int = 224) -> np.ndarray:
     return np.stack(imgs).astype(np.float32)
 
 
-def build_synthetic_hmr(seed: int, device="cpu"):
-    """tepose_b200.HMR (ResNet-50 + regressor) with make_hmr_state(seed) loaded, on `device`, in eval mode."""
+def build_synthetic_hmr(seed: int, device="cpu", precision: str = "bf16"):
+    """tepose_b200.HMR (ResNet-50 + regressor) of `precision` with make_hmr_state(seed) loaded, on `device`, in eval mode."""
     import tempfile
     import torch
     from .hmr import hmr
@@ -361,7 +361,7 @@ def build_synthetic_hmr(seed: int, device="cpu"):
         write_base_data(os.path.join(tmp, "data", "base_data"), seed)      # asset paths are cwd-relative
         os.chdir(tmp)
         try:
-            model = hmr(pretrained=False)
+            model = hmr(pretrained=False, precision=precision)
         finally:
             os.chdir(old)
     own = model.state_dict()

@@ -8,7 +8,8 @@ features go straight into the window's feature ring, and once the window is full
     crop -> HMR ResNet-50 (76 launches) -> feature roll -> TePose window step -> theta roll
 
 The window, both rings and the step body are tepose_b200.stream.WindowedTePose's.  The crop table is device memory read by the
-graph, so boxes may change on every frame.
+graph, so boxes may change on every frame.  With an HMR of precision "fp32_tc" the crop is written in split layout
+(tp_crop_normalize_split3) and the trunk runs on split-bf16 operands (HMR.features_nhwc12): fp32-grade features.
 
     vt = VideoTePose(hmr, model, model_vibe, J_regressor=J, batch=B)      # B tracked people (or B cameras)
     for frames, crops in video:                   # frames uint8 [F,H,W,3] RGB, crops [B,6] rows (frame, cx, cy, w, h, scale)
@@ -33,7 +34,7 @@ class VideoTePose:
         self.device, self.T = self.window.device, self.window.T
         self.use_graph = use_graph
         self.table = torch.zeros(batch, CROP_FIELDS, dtype=torch.int32, device=self.device)
-        self.x4 = torch.zeros(batch, CROP, CROP, 4, dtype=torch.bfloat16, device=self.device)
+        self.x4 = torch.zeros(batch, CROP, CROP, hmr.stem_channels, dtype=torch.bfloat16, device=self.device)   # the stem input
         self.frames = None                            # [F,H,W,3] uint8, allocated by the first push
         self.pushed = 0
         self.bootstrapped = False                     # VIBE has run on this clip
@@ -74,9 +75,11 @@ class VideoTePose:
     def _extract(self):
         """crop -> HMR -> the newest frame of the feature ring"""
         F, H, W, _ = self.frames.shape
-        nv.check(nv.lib().tp_crop_normalize_bf16(nv.ptr(self.frames), F, H, W, nv.ptr(self.table), self.B, nv.ptr(self.x4),
-                                                 nv.stream()), "tp_crop_normalize_bf16")
-        self.window.push_features(self.hmr.features_nhwc4(self.x4))
+        split = self.hmr.precision == "fp32_tc"
+        name = "tp_crop_normalize_split3" if split else "tp_crop_normalize_bf16"
+        nv.check(getattr(nv.lib(), name)(nv.ptr(self.frames), F, H, W, nv.ptr(self.table), self.B, nv.ptr(self.x4), nv.stream()),
+                 name)
+        self.window.push_features(self.hmr.features_nhwc12(self.x4) if split else self.hmr.features_nhwc4(self.x4))
 
     def _steady(self):
         self._extract()
