@@ -229,6 +229,25 @@ TP_API int tp_crop_normalize_bf16(const void* frames, int F, int H, int W, const
 TP_API int tp_crop_normalize_split3(const void* frames, int F, int H, int W, const tp_crop* crops, int N, void* out,
                                     void* stream);
 
+/* ------------------------------------------------------------------ tracked people: slot-managed windows
+ * The windowed loop's state x [S,T,ld] fp32 (ld >= 2133; frame t of slot s is the row x + (s*T + t)*ld: features in columns
+ * 0..2047, the theta ring in 2048..2132) for S slots, each holding one tracked person.  Two DEVICE tables of S int32 drive a
+ * push, read when the kernels run, so a captured graph follows tracks that start, pause and end between replays:
+ *   op[s]  0 = no frame for slot s this push, 1 = the next frame of the slot's track, 2 = the first frame of a new track;
+ *   src[s] the row of feats [>= S, 2048] fp32 holding slot s's frame.
+ * Rows are only 4-byte aligned (no 16-byte access is assumed).  The push leaves a slot whose op is outside {0,1,2} or whose
+ * src is outside [0,S) untouched and reads nothing for it; the commit (which reads no src) leaves a slot whose op is outside
+ * {0,1,2} untouched.  The callers validate the tables they write; a replayed graph cannot check them.  Every pointer 4-byte
+ * aligned. */
+/* Before the window step.  op 2: columns 0..2132 of every frame of the slot become 0, then feats[src[s]] is frame T-1;
+ * op 1: the slot's features shift one frame towards 0 and feats[src[s]] becomes frame T-1 (theta columns untouched);
+ * op 0: nothing. */
+TP_API int tp_window_slots_push(float* x, int S, int T, int64_t ld, const float* feats, const int32_t* src, const int32_t* op,
+                                void* stream);
+/* After the window step, with theta [S,85] fp32 its newest predictions: for op 1 or 2, theta ring [0..T-3] <- [1..T-2] and
+ * ring[T-2] <- theta[s] (evaluate.py:268-269 per slot); op 0 keeps the slot's ring.  Ring slot T-1 is never written. */
+TP_API int tp_window_slots_commit(float* x, int S, int T, int64_t ld, const float* theta, const int32_t* op, void* stream);
+
 /* ------------------------------------------------------------------ GRU recurrence (K2)
  * One direction of one torch.nn.GRU layer (lib/models/tepose.py:53-64,73,76) given the
  * input projections gi = x.W_ih^T + b_ih.  Step s (0-based) reads gi row block

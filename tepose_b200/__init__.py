@@ -5,6 +5,7 @@ from .vibe import VIBE  # noqa: F401
 from .spin import Regressor, projection  # noqa: F401
 from .hmr import HMR, hmr  # noqa: F401
 from .video import VideoTePose  # noqa: F401
+from .tracks import TrackedTePose, TrackedVideoTePose  # noqa: F401
 from .smpl import (SMPL, SMPLOutput, JOINT_MAP, JOINT_NAMES, JOINT_IDS, H36M_TO_J14, H36M_TO_J17,  # noqa: F401
                    SMPL_MODEL_DIR, SMPL_MEAN_PARAMS, BASE_DATA_DIR, get_smpl_faces)
 from .geometry import rot6d_to_rotmat, rotation_matrix_to_angle_axis, batch_rodrigues  # noqa: F401

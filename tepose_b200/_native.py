@@ -39,6 +39,7 @@ EXPORTS = [
     "tp_nchw_to_nhwc_bf16", "tp_im2col_nhwc_bf16", "tp_maxpool3x3s2_nhwc_bf16", "tp_avgpool_nhwc_bf16",
     "tp_crop_normalize_bf16",
     "tp_nchw_to_nhwc_split3", "tp_maxpool3x3s2_nhwc_split3", "tp_avgpool_nhwc_split3", "tp_crop_normalize_split3",
+    "tp_window_slots_push", "tp_window_slots_commit",
 ]
 
 vp, i32, i64, f32, sz = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
@@ -89,6 +90,8 @@ _SIGNATURES = {
     "tp_maxpool3x3s2_nhwc_split3": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]),
     "tp_avgpool_nhwc_split3": (C.c_int, [vp, vp, C.c_int, C.c_int, C.c_int, vp]),
     "tp_crop_normalize_split3": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, vp, C.c_int, vp, vp]),
+    "tp_window_slots_push": (C.c_int, [vp, C.c_int, C.c_int, i64, vp, vp, vp, vp]),
+    "tp_window_slots_commit": (C.c_int, [vp, C.c_int, C.c_int, i64, vp, vp, vp]),
     "tp_device_info": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(sz)]),
     "tp_rot6d_to_rotmat": (C.c_int, [vp, vp, i64, vp]),
     "tp_rotmat_to_angle_axis": (C.c_int, [vp, vp, i64, vp]),

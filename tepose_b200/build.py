@@ -12,7 +12,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtepose_b200.so")
 OBJ = os.path.join(HERE, "build")
-SOURCES = ["api.cu", "geometry.cu", "pack.cu", "gemm_f32.cu", "gemm_tc.cu", "skinny.cu", "gru.cu", "regressor.cu", "smpl.cu", "metrics.cu", "train.cu", "loss.cu", "conv.cu", "crop.cu"]
+SOURCES = ["api.cu", "geometry.cu", "pack.cu", "gemm_f32.cu", "gemm_tc.cu", "skinny.cu", "gru.cu", "regressor.cu", "smpl.cu", "metrics.cu", "train.cu", "loss.cu", "conv.cu", "crop.cu", "slots.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 
