@@ -210,8 +210,9 @@ class TemporalEncoder(nn.Module, GruKernels):
         """Runs K1 + K2.  Returns (h_fwd [B,H], h_rec [B,2H]) = (y[-1], y_rec[0]) of
         lib/models/tepose.py:73-80.  h0 = (hF0, hB0) carries state (live-stream mode, L=1);
         with return_states the per-step states (yF [T,B,H], yB [T,B,H]) of the two causal
-        directions are returned as well.  train_ctx (a dict, training path): the per-step states, the gate activations of every
-        step (tp_gru_job.gates) and an fp32 copy of the packed input are stored into it for the backward pass."""
+        directions are returned as well.  train_ctx (a dict, training path): per layer, the per-step states of every full
+        direction in its run order, the gate activations of every step (tp_gru_job.gates, indexed like the direction's
+        output) and the fp32 input of the layer are stored into train_ctx["layers"] for the backward pass."""
         nv.require_cuda(x, "input")
         if x.dim() != 3 or x.shape[2] != INPUT_SIZE:
             raise ValueError(f"expected input [B,T,{INPUT_SIZE}], got {tuple(x.shape)}")
@@ -236,9 +237,8 @@ class TemporalEncoder(nn.Module, GruKernels):
         seq_f = torch.empty(T, B, H, device=dev, dtype=torch.float32) if keep else None
         seq_b = torch.empty(T, B, H, device=dev, dtype=torch.float32) if keep else None
         gates_f = gates_b = gates_s = None
+        saved = []          # train_ctx["layers"]: one dict per layer
         if train_ctx is not None:
-            if Ln != 1:
-                raise NotImplementedError("training path: n_layers == 1 only")
             gates_f = torch.empty(T, B, 4 * H, device=dev, dtype=torch.float32)
             gates_b = torch.empty(T, B, 4 * H, device=dev, dtype=torch.float32)
             gates_s = torch.empty(1, B, 4 * H, device=dev, dtype=torch.float32)
@@ -260,9 +260,10 @@ class TemporalEncoder(nn.Module, GruKernels):
                         xp32 = torch.empty(T * B, kp, device=dev, dtype=torch.float32)
                         nv.check(L.tp_pack_rows(nv.vp(x.data_ptr()), x.stride(0), x.stride(1), B, T, INPUT_SIZE, nv.ptr(xp32), kp,
                                                 nv.PRECISION_FP32, 0, nv.stream()), "tp_pack_rows")
-                        train_ctx["xp"] = xp32
+                        x_in = xp32
                     else:
-                        train_ctx["xp"] = xp
+                        x_in = xp
+                    saved.append({"x": {"f": x_in, "r": x_in}})
                 if last:
                     gi = torch.empty(T * B, 6 * H, device=dev, dtype=torch.float32)      # [fwd | rec-backward]
                     gs = torch.empty(B, 3 * H, device=dev, dtype=torch.float32)          # rec-forward, newest frame only
@@ -301,6 +302,11 @@ class TemporalEncoder(nn.Module, GruKernels):
                 c_f = 0
                 # deeper layers of gru_rec are indexed by x_rec time tau: backward dir walks tau = T-1..0
                 f_in, b_in, s_in = (0, 1), (T - 1, -1), (0, 1)
+                if train_ctx is not None:         # the fp32 outputs of the layer below (zero-padded to kpf / kpr)
+                    saved.append({"x": {"f": y_f, "r": y_r}})
+            gl = [None, None, None]
+            if train_ctx is not None and not last:
+                gl = [torch.empty(T, B, 4 * H, device=dev, dtype=torch.float32) for _ in range(3)]
             if not last:
                 kpn_f, kpn_r = pk["layers"][l + 1]["kpf"], pk["layers"][l + 1]["kpr"]
                 ny_f = torch.zeros(T * B, kpn_f, device=dev, dtype=torch.float32)
@@ -328,17 +334,28 @@ class TemporalEncoder(nn.Module, GruKernels):
                 # outputs of gru_rec are stored by x_rec index tau: forward dir writes tau = s,
                 # backward dir writes tau = T-1-s
                 jobs = [
-                    self._job(dev, gi_f, c_f, w[0], b[0], T, f_in[0], f_in[1], y=ny_f, y_lp=ny_f_lp, w_umma=wu[0]),
+                    self._job(dev, gi_f, c_f, w[0], b[0], T, f_in[0], f_in[1], y=ny_f, y_lp=ny_f_lp, w_umma=wu[0], gates=gl[0]),
                     self._job(dev, gi_b, c_b, w[1], b[1], T, b_in[0], b_in[1], y=ny_r, ycol=H, y_lp=ny_r_lp,
-                              t_out0=T - 1, t_out_step=-1, w_umma=wu[1]),
-                    self._job(dev, gi_s, c_s, w[2], b[2], T, s_in[0], s_in[1], y=ny_r, ycol=0, y_lp=ny_r_lp, w_umma=wu[2]),
+                              t_out0=T - 1, t_out_step=-1, w_umma=wu[1], gates=gl[1]),
+                    self._job(dev, gi_s, c_s, w[2], b[2], T, s_in[0], s_in[1], y=ny_r, ycol=0, y_lp=ny_r_lp, w_umma=wu[2],
+                              gates=gl[2]),
                 ]
             self._recurrence(jobs, B, barrier=sync[l], precision=k2_prec)
             nv.mark(f"k2_recurrence_l{l}")
+            if train_ctx is not None:
+                if last:
+                    saved[l].update(seq={"f": seq_f, "b": seq_b}, gates={"f": gates_f, "b": gates_b, "s": gates_s})
+                else:
+                    # states in each direction's run order (the backward direction wrote tau = T-1-s); gates stay indexed
+                    # like the outputs
+                    st = lambda c0: ny_r[:, c0:c0 + H].reshape(T, B, H)
+                    saved[l].update(seq={"f": ny_f[:, :H].reshape(T, B, H).contiguous(), "b": st(H).flip(0).contiguous(),
+                                         "s": st(0).contiguous()},
+                                    gates={"f": gl[0], "b": gl[1], "s": gl[2]})
             if not last:
                 y_f, y_r, y_f_lp, y_r_lp = ny_f, ny_r, ny_f_lp, ny_r_lp
         if train_ctx is not None:
-            train_ctx.update(seq_f=seq_f, seq_b=seq_b, gates_f=gates_f, gates_b=gates_b, gates_s=gates_s)
+            train_ctx["layers"] = saved
         if return_states:
             return h_fwd, h_rec, seq_f, seq_b
         return h_fwd, h_rec

@@ -13,8 +13,11 @@ kernels; the backward is csrc/train.cu (SMPL / rotation / GRU-cell adjoints) + t
 Dropout masks are INPUTS (SURVEY.md H8): `forward(..., dropout_masks=m)` with m [n_iter, 2, 2B, 1024] in {0,1}; when omitted
 they are drawn with torch.rand on the device (what nn.Dropout does with its own generator).
 
-Scope: n_layers == 1 (the configuration BASELINE.json names); gradients flow to every encoder / regressor parameter, not to
-the input features.  `DataParallel` at the bottom is the one place of the package that uses a collective: one NCCL all-reduce
+Scope: any n_layers, including the released configuration (L = 2, H = 1024, T = 6) that every training config of the reference
+sets.  The backward walks the encoder top-down with one back-propagation-through-time loop for every (layer, direction): below
+the top layer, the gradient of a layer's output sequence is d_gi . W_ih of the layer above (one GEMM per upper direction) and
+is added to dL/dh before each step's cell adjoint.  Gradients flow to every encoder / regressor parameter, not to the input
+features.  `DataParallel` at the bottom is the one place of the package that uses a collective: one NCCL all-reduce
 per gradient bucket, launched from inside the backward as soon as a bucket is complete so that it overlaps the BPTT.
 """
 from __future__ import annotations
@@ -129,11 +132,12 @@ class TrainFunction(torch.autograd.Function):
 
 
 def path_parameters(model):
-    """The parameters the path reads, in a fixed order (regressor.smpl.* Parameters exist for state_dict parity only)."""
+    """The parameters the path reads, in a fixed order (regressor.smpl.* Parameters exist for state_dict parity only):
+    the twelve GRU tensors of every layer, the linear heads, the regressor."""
     enc, reg = model.encoder, model.regressor
-    names = ["gru_fwd.weight_ih_l0", "gru_fwd.weight_hh_l0", "gru_fwd.bias_ih_l0", "gru_fwd.bias_hh_l0",
-             "gru_rec.weight_ih_l0", "gru_rec.weight_hh_l0", "gru_rec.bias_ih_l0", "gru_rec.bias_hh_l0",
-             "gru_rec.weight_ih_l0_reverse", "gru_rec.weight_hh_l0_reverse", "gru_rec.bias_ih_l0_reverse", "gru_rec.bias_hh_l0_reverse"]
+    kinds = ("weight_ih", "weight_hh", "bias_ih", "bias_hh")
+    names = [f"gru_fwd.{k}_l{l}" for l in range(enc.n_layers) for k in kinds]
+    names += [f"gru_rec.{k}_l{l}{sfx}" for l in range(enc.n_layers) for sfx in ("", "_reverse") for k in kinds]
     out = []
     for n in names:
         mod, attr = n.split(".")
@@ -155,8 +159,6 @@ def make_dropout_masks(n_rows, device, n_iter=N_ITER, generator=None):
 def train_forward(model, x, dropout_masks=None):
     """lib/models/tepose.py:121-147 with is_train=True under .train(): list of one dict with [B, 2, ...] outputs attached to the
     autograd graph of the model's parameters."""
-    if model.encoder.n_layers != 1:
-        raise NotImplementedError("tepose_b200 training path: n_layers == 1 only (the configuration BASELINE.json names)")
     nv.require_cuda(x, "input")
     B = x.shape[0]
     if dropout_masks is None:
@@ -309,10 +311,14 @@ def _train_backward(model, sv, g_theta, g_verts, g_kp2d, g_kp3d, g_rotmat):
         _Ops.gemm(g_f, _Ops.transpose(f32(enc.linear_fwd.weight)), out=g_hcat[:, :H])
         _Ops.gemm(g_r, _Ops.transpose(f32(enc.linear_rec.weight)), out=g_hcat[:, H:])
         _Ops.relu_backward(g_hcat, h_cat)
+        layers = sv["layers"]
+        Ln = len(layers)
+        top = Ln - 1
         dbg = getattr(model, "_debug_capture", None)
         if dbg is not None:
-            dbg.update(g_hcat=g_hcat.clone(), h_cat=h_cat.clone(), g_feat=g_feat.clone(), seq_f=sv["seq_f"].clone(), seq_b=sv["seq_b"].clone(),
-                       gates_f=sv["gates_f"].clone(), gates_b=sv["gates_b"].clone())
+            dbg.update(g_hcat=g_hcat.clone(), h_cat=h_cat.clone(), g_feat=g_feat.clone(), seq_f=layers[top]["seq"]["f"].clone(),
+                       seq_b=layers[top]["seq"]["b"].clone(), gates_f=layers[top]["gates"]["f"].clone(),
+                       gates_b=layers[top]["gates"]["b"].clone())
         for name, g_rows, lo, hi in (("linear_fwd", g_f, 0, H), ("linear_rec", g_r, H, 3 * H)):
             dw = torch.empty(2048, hi - lo, device=dev, dtype=torch.float32)
             gT = _Ops.transpose(g_rows, B, 2048)
@@ -322,68 +328,127 @@ def _train_backward(model, sv, g_theta, g_verts, g_kp2d, g_kp3d, g_rotmat):
             grads[f"encoder.{name}.bias"] = _Ops.colsum(g_rows, B, 2048)
         if sync is not None:
             sync.ready([(k, grads[k]) for k in grads])                                 # regressor + heads: first bucket, overlaps the BPTT
-        # ---- GRU back-propagation through time: fwd direction, rec-backward direction (both over the original frame
-        #      order, only the final state is consumed: SURVEY.md F3) and the single step of the rec-forward direction
-        seq = {"f": sv["seq_f"], "b": sv["seq_b"]}
-        gates = {"f": sv["gates_f"], "b": sv["gates_b"], "s": sv["gates_s"]}
-        g_h = {"f": g_hcat[:, :H].contiguous(), "s": g_hcat[:, H:2 * H].contiguous(), "b": g_hcat[:, 2 * H:].contiguous()}
-        whhT = {"f": _Ops.transpose(f32(enc.gru_fwd.weight_hh_l0)), "b": _Ops.transpose(f32(enc.gru_rec.weight_hh_l0_reverse))}
+        # ---- GRU back-propagation through time, top layer first, over jobs (layer l, direction d): "f" = gru_fwd, "b" = the
+        #      reverse direction of gru_rec, "s" = the forward direction of gru_rec.  In the top layer only the final states
+        #      are consumed (SURVEY.md F3), and "s" is the single step at x_rec index 0 from h_0 = 0; below it every
+        #      direction is full and takes the gradient of its whole output sequence from the layer above.
+        def pname(l, d, k):
+            return f"encoder.gru_fwd.{k}_l{l}" if d == "f" else f"encoder.gru_rec.{k}_l{l}" + ("_reverse" if d == "b" else "")
+
+        def full(l):
+            return ("f", "b") if l == top else ("f", "b", "s")
+
+        def t_in(l, d, s):
+            """Row block of the layer's input that step s reads: layer 0 reads x in original frame order, deeper layers of
+            gru_rec read the x_rec-indexed sequence y_r (tau = T-1-t) of the layer below."""
+            if d == "f":
+                return s
+            if d == "b":
+                return s if l == 0 else T - 1 - s
+            if l == top:
+                return T - 1 if l == 0 else 0
+            return T - 1 - s if l == 0 else s
+
+        def t_out(l, d, s):
+            """Row block that step s writes of the output sequence (and of the saved gates)."""
+            return T - 1 - s if d == "b" and l != top else s
+
+        param = dict(model.named_parameters())
+        seq = {(l, d): layers[l]["seq"][d] for l in range(Ln) for d in full(l)}
+        gates = {(l, d): layers[l]["gates"][d] for l in range(Ln) for d in ("f", "b", "s")}
+        g_h = {(top, "f"): g_hcat[:, :H].contiguous(), (top, "s"): g_hcat[:, H:2 * H].contiguous(), (top, "b"): g_hcat[:, 2 * H:].contiguous()}
+        whhT = {(l, d): _Ops.transpose(f32(param[pname(l, d, "weight_hh")])) for l in range(top, -1, -1) for d in full(l)}
         # mixed precision (precision='bf16' models): the per-step dL/dh += d_gh . W_hh runs on the skinny tensor-core GEMM over a
         # fragment-packed bf16 copy of W_hh^T (25 MB streamed per step instead of 50 MB of fp32 through the FFMA GEMM)
         whh_lp = None
         if model.precision == "bf16" and B <= 64 and H % 16 == 0 and not getattr(model, "train_fp32_bptt", False):
-            whh_lp = {d: nv.pack_linear(whhT[d][:, :3 * H], "bf16") for d in ("f", "b")}
+            whh_lp = {j: nv.pack_linear(w[:, :3 * H], "bf16") for j, w in whhT.items()}
             sk_splits = 8                                  # 128-row groups x 8 K slices: 128 CTAs stream W_hh^T at H = 2048
             sk_ws = nv.workspace(int(L.tp_skinny_bf16_workspace_bytes(B, H, sk_splits)), dev)
             sk_ws[:4096].zero_()
-        dgi = {d: torch.empty(T * B, 3 * H, device=dev, dtype=torch.float32) for d in ("f", "b")}
-        dgh = {d: torch.empty(T * B, 3 * H, device=dev, dtype=torch.float32) for d in ("f", "b")}
-        dgi["s"] = torch.empty(B, 3 * H, device=dev, dtype=torch.float32)
-        dgh["s"] = torch.empty(B, 3 * H, device=dev, dtype=torch.float32)
+        # d_gi rows follow the layer's input (t_in), d_gh rows the run order (s)
+        dgi = {j: torch.empty(T * B, 3 * H, device=dev, dtype=torch.float32) for j in whhT}
+        dgh = {j: torch.empty(T * B, 3 * H, device=dev, dtype=torch.float32) for j in whhT}
+        dgi[(top, "s")] = torch.empty(B, 3 * H, device=dev, dtype=torch.float32)
+        dgh[(top, "s")] = torch.empty(B, 3 * H, device=dev, dtype=torch.float32)
 
-        def cell(d, s, hprev):
-            rows = slice(s * B, (s + 1) * B) if d != "s" else slice(0, B)
-            nv.check(L.tp_gru_cell_backward(P(g_h[d]), H, nv.vp(gates[d].data_ptr() + 4 * (0 if d == "s" else s * B * 4 * H)), 4 * H,
-                                            P(hprev), H, P(dgi[d][rows]), 3 * H, P(dgh[d][rows]), 3 * H, B, H, nv.stream()),
+        def cell(l, d, s):
+            j = (l, d)
+            single = j == (top, "s")
+            ri = slice(0, B) if single else slice(t_in(l, d, s) * B, (t_in(l, d, s) + 1) * B)
+            rh = slice(0, B) if single else slice(s * B, (s + 1) * B)
+            hprev = seq[j][s - 1] if s > 0 else None
+            nv.check(L.tp_gru_cell_backward(P(g_h[j]), H, nv.vp(gates[j].data_ptr() + 4 * t_out(l, d, s) * B * 4 * H), 4 * H,
+                                            P(hprev), H, P(dgi[j][ri]), 3 * H, P(dgh[j][rh]), 3 * H, B, H, nv.stream()),
                      "tp_gru_cell_backward")
 
-        cell("s", 0, None)
-        for s in range(T - 1, -1, -1):
-            for d in ("f", "b"):
-                cell(d, s, seq[d][s - 1] if s > 0 else None)
-                if s > 0 and whh_lp is not None:
-                    nv.check(L.tp_skinny_bf16(P(dgh[d][s * B:(s + 1) * B]), 3 * H, B, 3 * H, nv.ptr(whh_lp[d]), H, nv.vp(0), P(g_h[d]), H,
-                                              P(g_h[d]), H, 1.0, 1.0, 0, sk_splits, nv.ptr(sk_ws), sk_ws.numel(), nv.stream()), "tp_skinny_bf16")
-                elif s > 0:
-                    _Ops.gemm(dgh[d][s * B:(s + 1) * B], whhT[d], out=g_h[d], cin=g_h[d], beta=1.0)
+        for l in range(top, -1, -1):
+            dy = {}
+            if l < top:
+                # layer boundary: dL/d(outputs of layer l) = d_gi of layer l+1 . W_ih of layer l+1, one GEMM per upper direction
+                # over all T*B rows.  y_f [T*B, H] feeds "f" above; y_r [T*B, 2H] (columns [0,H) = this layer's "s",
+                # [H,2H) = its "b", rows by tau) feeds "b" and "s" above -- the top layer's "s" reads only tau = 0.
+                u = l + 1
+                wT = {d: _Ops.transpose(f32(param[pname(u, d, "weight_ih")])) for d in ("f", "b", "s")}
+                dy_f = _Ops.gemm(dgi[(u, "f")], wT["f"])
+                dy_r = _Ops.gemm(dgi[(u, "b")], wT["b"])
+                nr = dgi[(u, "s")].shape[0]
+                _Ops.gemm(dgi[(u, "s")], wT["s"], out=dy_r[:nr], cin=dy_r[:nr], beta=1.0)
+                dy = {"f": (dy_f, 0), "b": (dy_r, H), "s": (dy_r, 0)}
+                for d in full(l):
+                    g_h[(l, d)] = torch.empty(B, H, device=dev, dtype=torch.float32)
+            else:
+                cell(l, "s", 0)
+            for s in range(T - 1, -1, -1):
+                for d in full(l):
+                    j = (l, d)
+                    if dy:              # g_h += this step's output gradient (the first step of the walk starts from it)
+                        src, c0 = dy[d]
+                        r0 = t_out(l, d, s) * B
+                        nv.check(L.tp_axpby_f32(nv.vp(src.data_ptr() + 4 * (r0 * src.stride(0) + c0)), src.stride(0), P(g_h[j]), H, B, H,
+                                                1.0, 0.0 if s == T - 1 else 1.0, nv.stream()), "tp_axpby_f32")
+                    cell(l, d, s)
+                    if s > 0 and whh_lp is not None:
+                        nv.check(L.tp_skinny_bf16(P(dgh[j][s * B:(s + 1) * B]), 3 * H, B, 3 * H, nv.ptr(whh_lp[j]), H, nv.vp(0), P(g_h[j]), H,
+                                                  P(g_h[j]), H, 1.0, 1.0, 0, sk_splits, nv.ptr(sk_ws), sk_ws.numel(), nv.stream()), "tp_skinny_bf16")
+                    elif s > 0:
+                        _Ops.gemm(dgh[j][s * B:(s + 1) * B], whhT[j], out=g_h[j], cin=g_h[j], beta=1.0)
         if dbg is not None:
-            dbg.update(dgi_f=dgi["f"].clone(), dgi_b=dgi["b"].clone(), dgh_f=dgh["f"].clone(), dgh_b=dgh["b"].clone())
+            dbg.update(dgi_f=dgi[(top, "f")].clone(), dgi_b=dgi[(top, "b")].clone(), dgh_f=dgh[(top, "f")].clone(),
+                       dgh_b=dgh[(top, "b")].clone())
         # hidden-side weights: dW_hh = sum_t d_gh[t]^T h[t-1]  (rows B.. of d_gh against rows ..(T-1)B of the states)
-        names = {"f": "gru_fwd.{}_l0", "b": "gru_rec.{}_l0_reverse", "s": "gru_rec.{}_l0"}
         late = []
-        for d in ("f", "b"):
-            dw = torch.zeros(3 * H, H, device=dev, dtype=torch.float32)
-            if T > 1:
-                _Ops.weight_grad(dgh[d][B:], seq[d].reshape(T * B, H), dw, (T - 1) * B, tensor_core=tc)
-            grads["encoder." + names[d].format("weight_hh")] = dw
-            grads["encoder." + names[d].format("bias_hh")] = _Ops.colsum(dgh[d])
-            grads["encoder." + names[d].format("bias_ih")] = _Ops.colsum(dgi[d])
-            late += ["encoder." + names[d].format(k) for k in ("weight_hh", "bias_hh", "bias_ih")]
-        grads["encoder.gru_rec.weight_hh_l0"] = torch.zeros(3 * H, H, device=dev, dtype=torch.float32)   # h_0 = 0: no gradient reaches it
-        grads["encoder.gru_rec.bias_hh_l0"] = _Ops.colsum(dgh["s"])
-        grads["encoder.gru_rec.bias_ih_l0"] = _Ops.colsum(dgi["s"])
-        late += ["encoder.gru_rec.weight_hh_l0", "encoder.gru_rec.bias_hh_l0", "encoder.gru_rec.bias_ih_l0"]
+        for l in range(top, -1, -1):
+            for d in full(l):
+                j = (l, d)
+                dw = torch.zeros(3 * H, H, device=dev, dtype=torch.float32)
+                if T > 1:
+                    _Ops.weight_grad(dgh[j][B:], seq[j].reshape(T * B, H), dw, (T - 1) * B, tensor_core=tc)
+                grads[pname(l, d, "weight_hh")] = dw
+                grads[pname(l, d, "bias_hh")] = _Ops.colsum(dgh[j])
+                grads[pname(l, d, "bias_ih")] = _Ops.colsum(dgi[j])
+                late += [pname(l, d, k) for k in ("weight_hh", "bias_hh", "bias_ih")]
+            if l == top:
+                j = (top, "s")
+                grads[pname(top, "s", "weight_hh")] = torch.zeros(3 * H, H, device=dev, dtype=torch.float32)   # h_0 = 0: no gradient reaches it
+                grads[pname(top, "s", "bias_hh")] = _Ops.colsum(dgh[j])
+                grads[pname(top, "s", "bias_ih")] = _Ops.colsum(dgi[j])
+                late += [pname(top, "s", k) for k in ("weight_hh", "bias_hh", "bias_ih")]
         if sync is not None:
             sync.ready([(k, grads[k]) for k in late])
-        # input-side weights: dW_ih = d_gi^T X over all frames (the packed operand of K1 is reused)
-        xp = sv["xp"]                                                                  # [T*B, Kp] fp32, zero padded columns
-        F_in = enc.gru_fwd.weight_ih_l0.shape[1]
-        for d, rows0, nrows in (("f", 0, T * B), ("b", 0, T * B), ("s", (T - 1) * B, B)):
-            dw = torch.empty(3 * H, F_in, device=dev, dtype=torch.float32)
-            _Ops.weight_grad(dgi[d], xp[rows0:rows0 + nrows], dw, nrows, tensor_core=tc)
-            grads["encoder." + names[d].format("weight_ih")] = dw
-            if sync is not None:
-                sync.ready([("encoder." + names[d].format("weight_ih"), dw)])
+        # input-side weights: dW_ih = d_gi^T X over all frames (layer 0: the packed operand of K1; above: the fp32 outputs of
+        # the layer below; zero padded columns)
+        for l in range(top, -1, -1):
+            for d in ("f", "b", "s"):
+                j = (l, d)
+                x_in = layers[l]["x"]["f" if d == "f" else "r"]
+                rows0, nrows = (t_in(l, d, 0) * B, B) if j == (top, "s") else (0, T * B)
+                name = pname(l, d, "weight_ih")
+                dw = torch.empty(3 * H, param[name].shape[1], device=dev, dtype=torch.float32)
+                _Ops.weight_grad(dgi[j], x_in[rows0:rows0 + nrows], dw, nrows, tensor_core=tc)
+                grads[name] = dw
+                if sync is not None:
+                    sync.ready([(name, dw)])
     return [grads[name] for name, _ in path_parameters(model)]
 
 
