@@ -229,6 +229,28 @@ TP_API int tp_crop_normalize_bf16(const void* frames, int F, int H, int W, const
 TP_API int tp_crop_normalize_split3(const void* frames, int F, int H, int W, const tp_crop* crops, int N, void* out,
                                     void* stream);
 
+/* ------------------------------------------------------------------ demo output: mesh overlay
+ * The demo's overlay (lib/utils/renderer.py: Renderer.render, called once per person present, each over the previous result)
+ * with a contract of this library's own (tepose_b200/render.py, oracle/render_ref.py restate it):
+ *   - person i's vertex (X,Y,Z) of verts [n,V,3] fp32 lands at pixel u = (sx*(X+tx)+1)*W/2, v = (sy*(Y+ty)+1)*H/2 with
+ *     orig_cam[i] = (sx, sy, tx, ty) fp32 (the reference's weak-perspective camera with the mesh turned 180 degrees about x),
+ *     every fp32 operation separately rounded, snapped to 1/256 pixel; depth is Z, smaller nearer;
+ *   - a triangle with a non-finite vertex, a vertex more than 2^15 pixels from the origin, or zero snapped area draws nothing;
+ *   - pixel (x,y) is sampled at its centre; int64 edge functions with a top-left rule (both windings), so a pixel on an edge
+ *     shared by two triangles belongs to exactly one;
+ *   - visibility: later person first, then nearer, then lower face index (64-bit key: person 16 | depth 32 | face 16 bits);
+ *   - shading in float64: vertex normals are the normalised sums of the adjacent unit face normals in CSR order,
+ *     interpolated with the integer barycentrics and normalised; colour = colors[i] * (0.3 + 0.7*|n_z|), *255, clamped to
+ *     [0,255], rounded to nearest even.  Uncovered pixels copy the frame.
+ * frame, out uint8 [H,W,3] (frame is only read); colors [n,3] fp32; faces int32 [F,3]; vf_offsets int32 [V+1] and vf_faces
+ * int32 [vf_offsets[V]]: the faces of vertex v are vf_faces[vf_offsets[v] .. vf_offsets[v+1]) in ascending order.
+ * 0 <= n <= 65535, 1 <= F <= 65536, 1 <= H, W <= 32768.  workspace: tp_render_workspace_bytes(n, V, H, W) bytes, 16-byte
+ * aligned, any content (the first kernel resets what it reads).  Three kernels (project, raster, resolve), no host sync. */
+TP_API size_t tp_render_workspace_bytes(int n, int V, int H, int W);
+TP_API int tp_render_meshes(const void* frame, const float* verts, const float* orig_cam, const float* colors,
+                            const int32_t* faces, const int32_t* vf_offsets, const int32_t* vf_faces, int n, int V, int F,
+                            int H, int W, void* out, void* workspace, size_t workspace_bytes, void* stream);
+
 /* ------------------------------------------------------------------ tracked people: slot-managed windows
  * The windowed loop's state x [S,T,ld] fp32 (ld >= 2133; frame t of slot s is the row x + (s*T + t)*ld: features in columns
  * 0..2047, the theta ring in 2048..2132) for S slots, each holding one tracked person.  Two DEVICE tables of S int32 drive a
