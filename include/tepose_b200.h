@@ -270,6 +270,23 @@ TP_API int tp_window_slots_push(float* x, int S, int T, int64_t ld, const float*
  * ring[T-2] <- theta[s] (evaluate.py:268-269 per slot); op 0 keeps the slot's ring.  Ring slot T-1 is never written. */
 TP_API int tp_window_slots_commit(float* x, int S, int T, int64_t ld, const float* theta, const int32_t* op, void* stream);
 
+/* ------------------------------------------------------------------ demo output: pose smoothing
+ * The One-Euro filter of lib/utils/one_euro_filter.py as lib/utils/smooth_pose.py runs it (t_e = 1 on every row), as a
+ * ragged batched scan that carries its state between calls.  Sequence s of S filters its rows 0..count[s]-1 in order: row r of
+ * x is x + s*ld_seq_x + r*ld_row_x (C fp32 channels), and its result goes to the same place in out.  state [S,2,C] fp32 is
+ * x_prev | dx_prev per sequence.  With reset[s] != 0, row 0 is copied through unchanged and starts the state (x_prev = row 0,
+ * dx_prev = 0); otherwise filtering continues from state[s].  After the call state[s] holds the last row's x_hat | dx_hat.
+ * Per channel, with K = fl32(2*pi), every operation rounded on its own in fp32 (no FMA contraction):
+ *   a_d = K/(K+1);  dx = x - x_prev;  dx_hat = a_d*dx + (1-a_d)*dx_prev;  cutoff = min_cutoff + beta*|dx_hat|;
+ *   r = K*cutoff;  a = r/(r+1);  x_hat = a*x + (1-a)*x_prev
+ * which is bit-identical to the reference's float32 numpy arithmetic.  count and reset are DEVICE int32 [S], read when the
+ * kernel runs (a captured graph follows new tables); count[s] == 0, or outside [0,K], reads and writes nothing for sequence s.
+ * Strides >= C; rows need only 4-byte alignment (x may be the view theta[:, 3:75] of [N,85] rows).  min_cutoff and beta finite
+ * and >= 0.  One kernel, no host sync. */
+TP_API int tp_one_euro_filter(const float* x, int64_t ld_seq_x, int64_t ld_row_x, float* out, int64_t ld_seq_out,
+                              int64_t ld_row_out, float* state, const int32_t* count, const int32_t* reset, int S, int K, int C,
+                              float min_cutoff, float beta, void* stream);
+
 /* ------------------------------------------------------------------ GRU recurrence (K2)
  * One direction of one torch.nn.GRU layer (lib/models/tepose.py:53-64,73,76) given the
  * input projections gi = x.W_ih^T + b_ih.  Step s (0-based) reads gi row block

@@ -41,6 +41,7 @@ EXPORTS = [
     "tp_nchw_to_nhwc_split3", "tp_maxpool3x3s2_nhwc_split3", "tp_avgpool_nhwc_split3", "tp_crop_normalize_split3",
     "tp_window_slots_push", "tp_window_slots_commit",
     "tp_render_workspace_bytes", "tp_render_meshes",
+    "tp_one_euro_filter",
 ]
 
 vp, i32, i64, f32, sz = C.c_void_p, C.c_int32, C.c_int64, C.c_float, C.c_size_t
@@ -93,6 +94,7 @@ _SIGNATURES = {
     "tp_crop_normalize_split3": (C.c_int, [vp, C.c_int, C.c_int, C.c_int, vp, C.c_int, vp, vp]),
     "tp_window_slots_push": (C.c_int, [vp, C.c_int, C.c_int, i64, vp, vp, vp, vp]),
     "tp_window_slots_commit": (C.c_int, [vp, C.c_int, C.c_int, i64, vp, vp, vp]),
+    "tp_one_euro_filter": (C.c_int, [vp, i64, i64, vp, i64, i64, vp, vp, vp, C.c_int, C.c_int, C.c_int, f32, f32, vp]),
     "tp_render_workspace_bytes": (sz, [C.c_int, C.c_int, C.c_int, C.c_int]),
     "tp_render_meshes": (C.c_int, [vp, vp, vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, sz, vp]),
     "tp_device_info": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(sz)]),

@@ -31,6 +31,12 @@ those n rows and the trunk runs at the next power of two >= n (capped at S), one
     out = tv.push(frames [F,H,W,3] uint8, {track_id: (frame, cx, cy, w, h, scale)})
     res = tv.run(frames [N,H,W,3], {track_id: (frame_ids [n], boxes [n,5] (cx, cy, w, h, scale))})
 
+smooth=(min_cutoff, beta) adds the demo's pose smoothing (tepose_b200.smooth): each slot keeps One-Euro filter state on the
+device, a track's filter starts at its first output row and advances one row per push with output (a missed push leaves it
+as it is, as smooth_pose over the track's own rows does), and the filter and the SMPL run of the smoothed rows are part of the
+step graph, driven by two more rows of the slot table (count / reset, smooth_table).  Each output dict then also has
+pose_smooth [k,72], verts_smooth [k,6890,3] and joints3d_smooth [k,49,3]; the raw outputs do not change.
+
 The bookkeeping (SlotTable, bucket, compact_crops, schedule) is plain Python and runs without a GPU.
 """
 from __future__ import annotations
@@ -40,6 +46,7 @@ import torch
 
 from . import _native as nv
 from .hmr import CROP, CROP_FIELDS, make_crop_table
+from .smooth import POSE, SMOOTH_KEYS, one_euro_filter, smooth_params, smpl_rows
 from .stream import FEAT, OUTPUT_KEYS, WindowedTePose
 
 OP_NONE, OP_NEXT, OP_START = 0, 1, 2
@@ -115,6 +122,23 @@ class SlotTable:
         self.last = set()
 
 
+def smooth_table(plan: SlotPlan, S: int, T: int, bootstrap: bool):
+    """The per-slot filter table of a push with smoothing on: (count [S], reset [S]) for the filter of the step graph, and the
+    slots whose first T output rows (VIBE's T-1, then the first window's) the push filters eagerly.  A track's filter starts at
+    its first output row: at its T-th push, over T rows with a bootstrap model (eager) or over its one row without (in the
+    graph, reset); after that one row per push.  Absent tracks and tracks before their T-th push get count 0, which leaves the
+    slot's filter state as it is."""
+    count, reset, boot = [0] * S, [0] * S, []
+    for s, c in zip(plan.slots, plan.counts):
+        if c > T:
+            count[s] = 1
+        elif c == T and bootstrap:
+            boot.append(s)
+        elif c == T:
+            count[s], reset[s] = 1, 1
+    return count, reset, boot
+
+
 def bucket(n: int, slots: int) -> int:
     """The batch the HMR trunk runs at for n people present: the next power of two >= n, capped at `slots`."""
     if not 1 <= n <= slots:
@@ -160,13 +184,22 @@ def schedule(frames_by_track):
 
 # ---------------------------------------------------------------------------------------------------- features -> meshes
 class TrackedTePose:
-    def __init__(self, model, model_vibe=None, J_regressor=None, slots=1):
+    def __init__(self, model, model_vibe=None, J_regressor=None, slots=1, smooth=None):
+        """smooth=(min_cutoff, beta): also return each track's poses smoothed by the demo's One-Euro filter (tepose_b200.smooth)
+        and their meshes, as pose_smooth [k,72], verts_smooth [k,6890,3] and joints3d_smooth [k,49,3] next to the raw keys."""
+        self.smooth = smooth_params(smooth)
         self.table = SlotTable(slots)
         self.S = self.table.S
         self.window = WindowedTePose(model, model_vibe, J_regressor=J_regressor, batch=self.S)
         self.device, self.T = self.window.device, self.window.T
+        self.keys = OUTPUT_KEYS + (SMOOTH_KEYS if self.smooth else ())
         self.feats = torch.zeros(self.S, FEAT, device=self.device)                        # this push's features, src rows
-        self.tab = torch.zeros(2, self.S, dtype=torch.int32, device=self.device)          # [op; src]
+        # [op; src], and with smoothing [count; reset] of the step graph's filter (smooth_table)
+        self.tab = torch.zeros(4 if self.smooth else 2, self.S, dtype=torch.int32, device=self.device)
+        if self.smooth:
+            self.filter_state = torch.zeros(self.S, 2, POSE, device=self.device)         # x_prev | dx_prev per slot
+            self.pose_smooth = torch.zeros(self.S, POSE, device=self.device)
+            self.boot_tab = torch.zeros(2, self.S, dtype=torch.int32, device=self.device)  # count | reset of the bootstrap rows
         self.seed = {}                       # slot -> theta_input [T-1,85] given at the track's first push
         self._push_graph = self._step_graph = self._out = None
         self.launches_per_replay = None      # native launches of the push graph + the step graph
@@ -194,9 +227,33 @@ class TrackedTePose:
     def _step(self):
         win = self.window
         out = win.model(win.x, J_regressor=win.J_regressor)[-1]
-        nv.check(nv.lib().tp_window_slots_commit(nv.ptr(win.x), self.S, self.T, FEAT + 85, nv.ptr(out["theta"].contiguous()),
+        theta = out["theta"].contiguous()
+        nv.check(nv.lib().tp_window_slots_commit(nv.ptr(win.x), self.S, self.T, FEAT + 85, nv.ptr(theta),
                                                  nv.ptr(self.tab[0]), nv.stream()), "tp_window_slots_commit")
+        if self.smooth:
+            # one row per slot that has one this push (tab[2]); SMPL runs over all S rows, only those are returned
+            one_euro_filter(theta[:, 3:3 + POSE], self.pose_smooth, self.filter_state, self.tab[2], self.tab[3], 1, *self.smooth)
+            verts, joints = smpl_rows(self._smpl(), self.pose_smooth, theta[:, 75:85], self.S)
+            out = dict(out, pose_smooth=self.pose_smooth, verts_smooth=verts, joints3d_smooth=joints)
         return out
+
+    def _smpl(self):
+        return self.window.model.regressor.smpl
+
+    def _smooth_bootstrap(self, first, out, boot):
+        """The first T output rows of the slots in `boot` (VIBE's T-1 rows, then the window's), filtered from a reset state,
+        and their meshes: {slot: {key: [T,...]}}."""
+        S, T = self.S, self.T
+        theta = torch.cat([first["theta"], out["theta"][:, None]], 1)                    # [S,T,85]
+        cr = [[T if s in boot else 0 for s in range(S)], [1] * S]
+        self.boot_tab.copy_(torch.tensor(cr, dtype=torch.int32), non_blocking=True)
+        pose = torch.empty(S, T, POSE, device=self.device)
+        one_euro_filter(theta[:, :, 3:3 + POSE], pose, self.filter_state, self.boot_tab[0], self.boot_tab[1], T, *self.smooth)
+        idx = torch.tensor(boot, device=self.device)
+        p, b = pose[idx].reshape(-1, POSE), theta[idx, :, 75:85].reshape(-1, 10)
+        verts, joints = smpl_rows(self._smpl(), p, b, p.shape[0])
+        return {s: {"pose_smooth": pose[s], "verts_smooth": verts[j * T:(j + 1) * T], "joints3d_smooth": joints[j * T:(j + 1) * T]}
+                for j, s in enumerate(boot)}
 
     def _seeds(self, plan, theta_input):
         """theta_input {track id: [T-1,85]} for tracks that start at this push -> {slot: device tensor}."""
@@ -224,12 +281,19 @@ class TrackedTePose:
         self.seed.update(seeds)
         if not plan.ids:
             return {}
-        # a host table is pageable: the copy stages it before returning, so the next push cannot overwrite it in flight
-        self.tab.copy_(torch.tensor([plan.op, plan.src], dtype=torch.int32), non_blocking=True)
         win = self.window
+        rows = [plan.op, plan.src]
+        if self.smooth:
+            count, reset, smooth_boot = smooth_table(plan, self.S, self.T, win.vibe is not None)
+            rows += [count, reset]
+        # a host table is pageable: the copy stages it before returning, so the next push cannot overwrite it in flight
+        self.tab.copy_(torch.tensor(rows, dtype=torch.int32), non_blocking=True)
         if self._push_graph is None:
             self._push_graph, _, n_push = win._capture(self._push_kernel)
+            keep = self.filter_state.clone() if self.smooth else None
             self._step_graph, self._out, n_step = win._capture(self._step)
+            if self.smooth:                  # the capture's warm-up run advanced the filter state too
+                self.filter_state.copy_(keep)
             self.launches_per_replay = n_push + n_step
         self._push_graph.replay()
         boot = [s for s, c in zip(plan.slots, plan.counts) if c == self.T]
@@ -241,12 +305,14 @@ class TrackedTePose:
                 win.theta_input[s].copy_(self.seed[s] if s in self.seed else first["theta"][s])
         self._step_graph.replay()
         out = self._out
+        booted = self._smooth_bootstrap(first, out, smooth_boot) if self.smooth and smooth_boot else {}
         res = {}
         for i, s, c in zip(plan.ids, plan.slots, plan.counts):
             if c > self.T or (c == self.T and first is None):
-                res[i] = {k: out[k][s:s + 1] for k in OUTPUT_KEYS}
+                res[i] = {k: out[k][s:s + 1] for k in self.keys}
             elif c == self.T:
                 res[i] = {k: torch.cat([first[k][s], out[k][s:s + 1]], 0) for k in OUTPUT_KEYS}
+                res[i].update(booted.get(s, {}))
         return res
 
     @torch.no_grad()
@@ -267,11 +333,12 @@ class TrackedTePose:
 
     # ------------------------------------------------------------------ whole clip
     @torch.no_grad()
-    def run(self, features_by_track, theta_input=None, keys=OUTPUT_KEYS):
+    def run(self, features_by_track, theta_input=None, keys=None):
         """features_by_track {id: (first frame or frame ids [n], feats [n,2048])}: frame ids strictly increasing, gaps meaning
         the person was missed.  Returns {id: {key: [n,...]}} for the tracks with at least T frames: each track's outputs as
         WindowedTePose.run gives them for its own frames (frames 0..T-2 from VIBE; NaN without a bootstrap model).
-        theta_input {id: [T-1,85]} seeds those tracks' rings.  Every slot is freed first, and each track after its last frame."""
+        theta_input {id: [T-1,85]} seeds those tracks' rings.  Every slot is freed first, and each track after its last frame.
+        keys: the outputs to collect (default: every key a push returns, the smoothed ones included when smoothing is on)."""
         frames, feats = {}, {}
         for i, (spec, f) in features_by_track.items():
             f = torch.as_tensor(f)
@@ -284,10 +351,11 @@ class TrackedTePose:
 
 def _run_clip(owner, frames, push, theta_input, keys):
     """The per-person loop of a whole clip: frames {id: frame ids [n]}; push(frame, [(id, index)], theta_input) -> the push's
-    outputs.  Returns {id: {key: [n,...]}}."""
+    outputs.  Returns {id: {key: [n,...]}} for `keys` (None: owner.keys)."""
     unknown = set(theta_input or {}) - set(frames)
     if unknown:
         raise ValueError(f"theta_input for unknown tracks {sorted(map(repr, unknown))}")
+    keys = owner.keys if keys is None else keys
     owner.reset()
     res = {}
     for f, present, ending in schedule(frames):
@@ -309,13 +377,17 @@ def _run_clip(owner, frames, push, theta_input, keys):
 
 # ---------------------------------------------------------------------------------------------------- frames -> meshes
 class TrackedVideoTePose:
-    def __init__(self, hmr, model, model_vibe=None, J_regressor=None, slots=1):
+    def __init__(self, hmr, model, model_vibe=None, J_regressor=None, slots=1, smooth=None):
         nv.require_cuda(next(hmr.parameters()), "HMR parameters")
         self.hmr = hmr
-        self.tracker = TrackedTePose(model, model_vibe, J_regressor=J_regressor, slots=slots)
+        self.tracker = TrackedTePose(model, model_vibe, J_regressor=J_regressor, slots=slots, smooth=smooth)
         self.device, self.T, self.S = self.tracker.device, self.tracker.T, self.tracker.S
         self.frames = None                   # [F,H,W,3] uint8, allocated by the first push
         self.buckets = {}                    # trunk batch -> {table, extract, graph, launches}
+
+    @property
+    def keys(self):
+        return self.tracker.keys
 
     def end(self, track_id) -> None:
         self.tracker.end(track_id)
@@ -374,7 +446,7 @@ class TrackedVideoTePose:
         return self.tracker._advance(plan, seeds)
 
     @torch.no_grad()
-    def run(self, frames: torch.Tensor, tracks, theta_input=None, keys=OUTPUT_KEYS):
+    def run(self, frames: torch.Tensor, tracks, theta_input=None, keys=None):
         """frames uint8 [N,H,W,3]; tracks {id: (frame ids [n], boxes [n,5] rows (cx, cy, w, h, scale))}, frame ids strictly
         increasing in [0, N) (gaps: the person was missed).  Returns {id: {key: [n,...]}} as TrackedTePose.run does on the
         features of those crops."""
